@@ -250,6 +250,8 @@ class Job(object):
         self.fetched = [(torch.full((1,), float("nan")).pin_memory(), torch.full((2,), -1, dtype=torch.int64).pin_memory())
                         for _ in range(64)]
         self.fetch_i = 0
+        self.keep_last = False  # --dump-outputs: hold on to what this step hands back to its caller
+        self.last = None
 
     def step(self, b, fetch=False, comm=True):
         from ctc_pytorch_b200 import ops
@@ -268,6 +270,8 @@ class Job(object):
         self.opt.zero_grad(set_to_none=True)
         loss.backward()        # with grad_sync set, the per-layer all-reduces are launched and joined inside the backward pass
         self.opt.step()
+        if self.keep_last:
+            self.last = {"loss": loss, "log_probs": out, "greedy_labels": labels, "greedy_lengths": lens, "edit_distance": dist_}
         if fetch:
             # device -> host read of this step's result into pinned memory, every step, without stalling the launch queue — the
             # policy of the product's epoch loop (ctc_pytorch_b200/train.py run_epoch: device-side accumulation, no per-step
@@ -283,7 +287,7 @@ class Job(object):
 PER_STEP = None   # list of per-step event times of every timed loop when --per-step is given
 
 
-def timed_loop(job, steps, flush, world, e2e):
+def timed_loop(job, steps, flush, world, e2e, keep_last=False):
     import torch.distributed as dist
 
     def barrier():
@@ -301,6 +305,7 @@ def timed_loop(job, steps, flush, world, e2e):
             job.step(b, fetch=True)
         else:
             flush.zero_()  # L2 flush between steps (counted inside the timed region: ~0.03 ms)
+            job.keep_last = keep_last and k == steps - 1   # only the final step's results are held (--dump-outputs)
             job.step(job.devb[k % len(job.devb)])
         if marks is not None:
             marks[k].record()
@@ -317,6 +322,46 @@ def timed_loop(job, steps, flush, world, e2e):
     if world > 1:
         dist.all_reduce(ms, op=dist.ReduceOp.MAX)
     return float(ms.item())
+
+
+DUMP_SAMPLE = 1 << 16          # entries kept of each parameter-sized tensor
+DUMP_LIMIT = 64 * 1024 * 1024  # bytes written in all
+
+
+def dump_outputs(job, path):
+    """Writes what the last step of `job` handed back to its caller as <path>/<name>.npy (float32, or float64 for the loss
+    and the integer results): the loss, the log-probs, the greedy decode and its edit distances, and the state the step left
+    behind, i.e. every parameter's gradient, every parameter after the optimizer step and the BatchNorm running statistics.
+    Tensors with more than DUMP_SAMPLE entries are reduced to a fixed sample whose positions are seeded by the tensor's name,
+    so that two builds of the project can be compared array for array."""
+    import zlib
+    import numpy as np
+
+    def sample(name, t):
+        flat = t.detach().reshape(-1)
+        if flat.numel() <= DUMP_SAMPLE:
+            return flat
+        rng = np.random.default_rng(zlib.crc32(name.encode()))
+        idx = np.sort(rng.choice(flat.numel(), DUMP_SAMPLE, replace=False))
+        return flat[torch.from_numpy(idx).to(flat.device)]
+
+    last = job.last
+    arrays = {"loss": last["loss"].detach().double().reshape(1), "log_probs": last["log_probs"].detach().float()}
+    for k in ("greedy_labels", "greedy_lengths", "edit_distance"):
+        arrays[k] = last[k].double()
+    for k, p in job.model.named_parameters():
+        arrays["grad." + k] = sample("grad." + k, p.grad).float()
+        arrays["param." + k] = sample("param." + k, p).float()
+    for k, b in job.model.named_buffers():
+        if b.is_floating_point():
+            arrays["buffer." + k] = sample("buffer." + k, b).float()
+    arrays = {k: v.cpu().numpy() for k, v in arrays.items()}
+    total = sum(a.nbytes for a in arrays.values())
+    if total > DUMP_LIMIT:
+        raise RuntimeError("--dump-outputs: %d bytes exceed the %d byte limit" % (total, DUMP_LIMIT))
+    os.makedirs(path, exist_ok=True)
+    for k, a in arrays.items():
+        np.save(os.path.join(path, k + ".npy"), a)
 
 
 def run_ours(args, name, cfg, rank, world):
@@ -342,9 +387,14 @@ def run_ours(args, name, cfg, rank, world):
     # ---- timed region 1: inputs resident in HBM ----
     sampler.open_window()
     launches0 = L.launches
-    ms_dev = timed_loop(job, args.steps, flush, world, e2e=False)
+    ms_dev = timed_loop(job, args.steps, flush, world, e2e=False, keep_last=bool(args.dump_outputs))
     launches = L.launches - launches0
     sampler.close_window()
+    if args.dump_outputs:
+        job.keep_last = False
+        if rank == 0:
+            dump_outputs(job, args.dump_outputs)
+        job.last = None
     # ---- timed region 2: end to end from host buffers ----
     sampler.open_window()
     ms_e2e = timed_loop(job, args.steps, flush, world, e2e=True)
@@ -359,7 +409,7 @@ def run_ours(args, name, cfg, rank, world):
         job.model.precision = alt
         for w in range(3):
             job.step(job.devb[w % len(job.devb)])
-        k_alt = max(3, min(args.steps, 6))
+        k_alt = args.steps
         ms_alt = timed_loop(job, k_alt, flush, world, e2e=False)
         job.model.precision = args.precision
         other_precision = {"precision": alt, "ms_per_step": ms_alt / k_alt, "value": job.n_global * k_alt / (ms_alt * 1e-3),
@@ -370,7 +420,7 @@ def run_ours(args, name, cfg, rank, world):
         job4 = Job("cfg4", c4, rank, world, dev, args.precision, True, n_batches=2)
         for w in range(3):
             job4.step(job4.devb[w % 2])
-        k4 = max(3, min(args.steps, 5))
+        k4 = args.steps
         ms4 = timed_loop(job4, k4, flush, world, e2e=False)
         strong_line = {"config": workload_name("cfg4", c4, job4.n_local), "scaling": "strong", "global_batch": c4["N"],
                        "per_gpu_batch": job4.n_local, "n_gpus": world, "steps": k4, "ms_per_step": ms4 / k4,
@@ -394,7 +444,7 @@ def run_ours(args, name, cfg, rank, world):
         per_call.setdefault(nm, []).append((s, e))
         return r
     L.call = timed_call
-    prof_steps = 3
+    prof_steps = args.steps
     overlap_was, gx_was, dg_was = job.model.overlap_wgrad, job.model.overlap_gx, job.model.overlap_dg
     # kernels timed one at a time on one stream (the timed steps above overlap the wgrad GEMMs with BPTT and stream the input
     # projection under the forward recurrence)
@@ -545,7 +595,13 @@ def main():
     ap.add_argument("--no-cpu-baseline", action="store_true")
     ap.add_argument("--per-step", dest="per_step", action="store_true",
                     help="diagnostic: also record the device time of every step of the timed loops (key per_step_ms)")
+    ap.add_argument("--dump-outputs", dest="dump_outputs", default=None, metavar="DIR",
+                    help="after the timed steps, write what the last one computed as DIR/<name>.npy (see dump_outputs)")
     args = ap.parse_args()
+    if args.steps < 1:
+        ap.error("--steps must be at least 1")
+    if args.dump_outputs and args.impl != "ours":
+        ap.error("--dump-outputs applies to --impl ours")
     if args.per_step:
         global PER_STEP
         PER_STEP = []

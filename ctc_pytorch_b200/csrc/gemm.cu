@@ -20,6 +20,9 @@
 //   warps 4-7 epilogue: tcgen05.ld 32 lanes x 32 columns per warp, convert, store to global; the
 //             second accumulator buffer lets the next tile's MMAs run under the stores.
 #include <cstdlib>
+#include <map>
+#include <mutex>
+#include <utility>
 
 #include "common.cuh"
 #include "ctcb200.h"
@@ -45,7 +48,8 @@ template <int BN>
 __global__ void __launch_bounds__(256, 1)
 gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ CUtensorMap tmB,
                const __grid_constant__ CUtensorMap tmC, void* __restrict__ Cout, long long ldc, int M, int N, int K,
-               int a_koff, int b_koff, int out_bf16, int accumulate, int tma_store, int split_k, int mn_major) {
+               int a_koff, int b_koff, int out_bf16, int accumulate, int tma_store, int split_k, int mn_major,
+               unsigned int* __restrict__ split_turn, unsigned int ticket_base) {
     using Cfg = GemmCfg<BN>;
     constexpr int STAGES = Cfg::STAGES;
     extern __shared__ uint8_t smem_raw[];
@@ -81,16 +85,22 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         fence_mbar_init();
     }
     if (warp == 2) tmem_alloc(tmem_slot, Cfg::TMEM_COLS);
+    // split_k > 1: every CTA owns one work item, handed out in the order the CTAs start (a ticket counter in
+    // split_turn[0] that keeps counting across the launches of a stream; ticket_base is where this launch began).
+    // A split then only ever waits for splits whose CTAs are already running, whatever order blocks are dispatched in.
+    uint32_t* first_tile = tmem_slot + 1;
+    if (threadIdx.x == 0) *first_tile = split_k > 1 ? atomicAdd(split_turn, 1u) - ticket_base : blockIdx.x;
     tc_fence_before();
     __syncthreads();
     tc_fence_after();
     const uint32_t tmem_base = *tmem_slot;
+    const int tile0 = static_cast<int>(*first_tile);
 
     if (warp == 0) {
         if (lane == 0) {
             int stage = 0;
             uint32_t phase = 0;
-            for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x) {
+            for (int tile = tile0; tile < tiles; tile += gridDim.x) {
                 const int ot = tile % out_tiles, sp = tile / out_tiles;
                 const int m_blk = ot % m_tiles, n_blk = ot / m_tiles;
                 const int kb0 = sp * kb_per_split, kb1 = min(kblocks_total, kb0 + kb_per_split);
@@ -125,7 +135,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         int stage = 0;
         uint32_t phase = 0;
         int it = 0;
-        for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
+        for (int tile = tile0; tile < tiles; tile += gridDim.x, ++it) {
             const int acc = it & 1;
             const uint32_t acc_phase = (it >> 1) & 1;
             mbar_wait(&tempty[acc], acc_phase ^ 1);
@@ -161,7 +171,7 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
         __nv_bfloat16* Cb = reinterpret_cast<__nv_bfloat16*>(Cout);
         const bool vec_f32 = (ldc % 4 == 0) && ((reinterpret_cast<uintptr_t>(Cout) & 15) == 0);
         const bool vec_b16 = (ldc % 8 == 0) && ((reinterpret_cast<uintptr_t>(Cout) & 15) == 0);
-        for (int tile = blockIdx.x; tile < tiles; tile += gridDim.x, ++it) {
+        for (int tile = tile0; tile < tiles; tile += gridDim.x, ++it) {
             const int ot = tile % out_tiles;
             const int m_blk = ot % m_tiles, n_blk = ot / m_tiles;
             const int acc = it & 1;
@@ -176,6 +186,18 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                 uint8_t* wbuf = staging + ew * 8192;
                 const int sp = tile / out_tiles;
                 const bool has_work = sp * kb_per_split < kblocks_total;  // an empty K split contributes nothing
+                // K splits add their partial tiles into C one after another in split order (a turn counter per output
+                // tile and epilogue warp), so the float sums, and with them the result, are the same on every run.
+                // Split sp waits only for splits that took lower tickets, i.e. CTAs that are already running.
+                unsigned int* turn = split_k > 1 ? split_turn + 1 + ot * 4 + ew : nullptr;
+                if (turn) {
+                    if (lane == 0) {
+                        while (ld_acquire(turn) != static_cast<unsigned int>(sp)) {
+                        }
+                        fence_proxy_async_all();
+                    }
+                    __syncwarp();
+                }
 #pragma unroll 1
                 for (int c0 = 0; c0 < BN; c0 += 32) {
                     const int col0 = n_blk * BN + c0;
@@ -197,6 +219,12 @@ gemm_tn_kernel(const __grid_constant__ CUtensorMap tmA, const __grid_constant__ 
                         else tma_store_2d(&tmC, box, col0, m_blk * BM + ew * 32);
                         bulk_group_commit();
                     }
+                }
+                if (turn && lane == 0) {   // this split's additions are complete in global memory: pass the turn on
+                    bulk_group_wait_all();
+                    fence_proxy_async_all();
+                    if (sp == split_k - 1) *turn = 0u;   // the last split leaves the counter zeroed for the next launch
+                    else red_release_add(turn, 1u);
                 }
                 tc_fence_before();
                 __syncwarp();
@@ -291,7 +319,7 @@ int gemm_prepare() {
 template <int BN>
 int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMap& tmC, int tma_store, int split_k,
                 void* C, long long ldc, int M, int N, int K, int a_koff, int b_koff, int out_bf16, int accumulate,
-                int max_ctas, cudaStream_t stream, int mn_major = 0) {
+                int max_ctas, cudaStream_t stream, int mn_major, unsigned int* split_turn, unsigned int ticket_base) {
     using Cfg = GemmCfg<BN>;
     const int rc_attr = gemm_prepare<BN>();
     if (rc_attr != OK) return rc_attr;
@@ -300,13 +328,39 @@ int launch_gemm(const CUtensorMap& tmA, const CUtensorMap& tmB, const CUtensorMa
     // (short-lived CTAs, so a kernel launched later on another stream gets SMs quickly)
     int limit = max_ctas > 0 ? max_ctas : device_sm_count();
     int grid = (max_ctas < 0 || tiles < limit) ? tiles : limit;
+    CTCB_REQUIRE(split_k == 1 || grid == tiles, "gemm: a split-K launch needs one CTA per work item (%d tiles, grid %d)", tiles, grid);
     gemm_tn_kernel<BN><<<grid, 256, Cfg::SMEM_BYTES, stream>>>(tmA, tmB, tmC, C, ldc, M, N, K, a_koff, b_koff, out_bf16,
-                                                              accumulate, tma_store, split_k, mn_major);
+                                                              accumulate, tma_store, split_k, mn_major, split_turn,
+                                                              ticket_base);
     CTCB_LAUNCH_CHECK();
     return OK;
 }
 
 }  // namespace
+
+// Ordered split-K additions, one state per (device, stream): a buffer of 1 + device_sm_count() * 4 words (the ticket
+// counter, then the turn counters: a split launch has at most sms / 2 output tiles, 4 epilogue warps each), zeroed once
+// when the stream first runs a split launch, and the ticket count the stream's launches have taken so far. Every launch
+// leaves its turn counters at zero, so the launches of one stream reuse the buffer; launches in different streams, which
+// may run concurrently, never share one.
+struct SplitState {
+    unsigned int* buf = nullptr;
+    unsigned int tickets = 0;
+};
+static std::mutex split_mu;
+static std::map<std::pair<int, cudaStream_t>, SplitState> split_states;
+
+static int split_state(cudaStream_t stream, SplitState** out) {
+    std::lock_guard<std::mutex> lock(split_mu);
+    SplitState& st = split_states[std::make_pair(current_device(), stream)];
+    if (!st.buf) {
+        const size_t bytes = (1 + static_cast<size_t>(device_sm_count()) * 4) * sizeof(unsigned int);
+        CTCB_CUDA(cudaMalloc(reinterpret_cast<void**>(&st.buf), bytes));
+        CTCB_CUDA(cudaMemsetAsync(st.buf, 0, bytes, stream));
+    }
+    *out = &st;
+    return OK;
+}
 
 // Internal entry used by the other translation units as well as the C ABI below.
 static int gemm_impl(const void* A, long long lda, const void* B, long long ldb, void* C, long long ldc, int M, int N,
@@ -364,11 +418,23 @@ static int gemm_impl(const void* A, long long lda, const void* B, long long ldb,
         while (split_k < 8 && t * (split_k * 2) <= sms && kblocks / (split_k * 2) >= 16) split_k *= 2;
         if (split_k > 1 && !accumulate) CTCB_CUDA(cudaMemsetAsync(C, 0, static_cast<size_t>(M) * ldc * sizeof(float), stream));
     }
-    switch (bn) {
-        case 64: return launch_gemm<64>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major);
-        case 128: return launch_gemm<128>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major);
-        default: return launch_gemm<256>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major);
+    SplitState* st = nullptr;
+    if (split_k > 1) {
+        rc = split_state(stream, &st);
+        if (rc != OK) return rc;
     }
+    unsigned int* split_turn = st ? st->buf : nullptr;
+    const unsigned int base = st ? st->tickets : 0u;
+    switch (bn) {
+        case 64: rc = launch_gemm<64>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major, split_turn, base); break;
+        case 128: rc = launch_gemm<128>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major, split_turn, base); break;
+        default: rc = launch_gemm<256>(tmA, tmB, tmC, tma_store, split_k, C, ldc, M, N, K, a_koff, b_koff, out_bf16, accumulate, max_ctas, stream, mn_major, split_turn, base); break;
+    }
+    if (rc == OK && st) {   // the launch's CTAs take exactly its tile count of tickets (one work item per CTA)
+        std::lock_guard<std::mutex> lock(split_mu);
+        st->tickets = base + static_cast<unsigned int>(m_tiles * ((N + bn - 1) / bn) * split_k);
+    }
+    return rc;
 }
 
 int gemm_preload() {

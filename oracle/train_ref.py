@@ -57,3 +57,22 @@ def schedule_trace(dev_losses, accs, init_lr, decay, end_adjust_acc, num_epoches
             ev["stop"] = True
         trace.append(ev)
     return trace, {"loss_best": loss_best, "acc_best": acc_best, "epochs": count}
+
+
+def scripted_sequence(seed, n):
+    """Seeded per-epoch (dev loss, accuracy) sequence mixing improvements, plateaus inside the +-end_adjust_acc band and
+    divergences, so that every branch of the policy is exercised."""
+    import random
+    rng = random.Random(seed)
+    loss, out_l, out_a = 40.0 + rng.random() * 10, [], []
+    for i in range(n):
+        r = rng.random()
+        if r < 0.45:
+            loss -= rng.random() * 2.0          # clear improvement
+        elif r < 0.8:
+            loss += (rng.random() - 0.5) * 0.02  # plateau inside the +-end_adjust_acc band
+        else:
+            loss += rng.random() * 3.0          # divergence -> immediate halving
+        out_l.append(loss)
+        out_a.append(rng.random())
+    return out_l, out_a

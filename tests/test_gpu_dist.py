@@ -63,7 +63,7 @@ def _rank_main(rank, world, port, out, precision):
 @pytest.mark.parametrize("precision", ["bf16", "x3"])
 def test_two_rank_gradients_equal_mean_of_per_shard_oracle(tmp_path, precision):
     if not torch.cuda.is_available() or torch.cuda.device_count() < 2:
-        pytest.skip("needs two CUDA devices (run with gpurun --gpus 2)")
+        pytest.skip("needs two CUDA devices")
     import torch.multiprocessing as mp
     from ctc_pytorch_b200.dist import shard_range
     world = 2

@@ -441,6 +441,67 @@ def test_model_vs_oracle(T, N, F, H, L, C, bn, tile):
         assert relnorm(p.grad, rp[k].grad) < 3e-2, (k, relnorm(p.grad, rp[k].grad))
 
 
+def test_split_k_gemm_is_bitwise_repeatable():
+    """Weight-gradient shapes (short-fat output, long K) are split along K; the splits add into C in split order, so repeated
+    calls, with and without accumulation and on two streams at once, give identical bits."""
+    from ctc_pytorch_b200 import ops
+    g = torch.Generator().manual_seed(3)
+    K, M, N = 8192, 512, 256
+    a = torch.randn(K, M, generator=g).to(DEV, torch.bfloat16)
+    b = torch.randn(K, N, generator=g).to(DEV, torch.bfloat16)
+    c0 = torch.randn(M, N, generator=g).to(DEV)
+    first = ops.gemm_atb(a, b)
+    want = a.double().t() @ b.double()
+    assert relnorm(first, want) < 1e-5
+    acc_first = ops.gemm_atb(a, b, out=c0.clone(), accumulate=True)
+    side = torch.cuda.Stream()
+    for _ in range(3):
+        side.wait_stream(torch.cuda.current_stream())
+        with torch.cuda.stream(side):
+            on_side = ops.gemm_atb(a, b)
+        on_main = ops.gemm_atb(a, b)
+        acc = ops.gemm_atb(a, b, out=c0.clone(), accumulate=True)
+        torch.cuda.current_stream().wait_stream(side)
+        torch.cuda.synchronize()
+        assert torch.equal(on_side, first) and torch.equal(on_main, first) and torch.equal(acc, acc_first)
+
+
+def test_training_step_is_bitwise_repeatable():
+    """One training step (forward, CTC loss, backward with the side-stream weight gradients, fused Adam) repeated from the same
+    state gives identical log-probs, loss, gradients and updated parameters."""
+    import copy
+    from ctc_pytorch_b200.model import CTC_Model
+    from ctc_pytorch_b200.loss import CTCLoss
+    torch.manual_seed(0)
+    T, N, F, H, L, C = 200, 16, 40, 512, 2, 62
+    rnn_param = {"rnn_input_size": F, "rnn_hidden_size": H, "rnn_layers": L, "rnn_type": nn.LSTM, "bidirectional": True,
+                 "batch_norm": True}
+    m = CTC_Model(rnn_param=rnn_param, num_class=C, drop_out=0.0).to(DEV)
+    opt = torch.optim.Adam(m.parameters(), lr=1e-3, weight_decay=0.005, fused=True)
+    x, frac, tg, tl = model_ref.synthetic_batch(T, N, F, C, 30, 2)
+    x, tg, tl = x.to(DEV), tg.to(DEV), tl.to(DEV)
+    il = (frac * T).long().to(DEV)
+    m.train()
+    sd, osd = copy.deepcopy(m.state_dict()), copy.deepcopy(opt.state_dict())
+
+    def step():
+        m.load_state_dict(sd)
+        opt.load_state_dict(osd)
+        out = m(x)
+        loss = CTCLoss(reduction="sum")(out, tg, il, tl) / N
+        opt.zero_grad(set_to_none=True)
+        loss.backward()
+        opt.step()
+        torch.cuda.synchronize()
+        return ([("log_probs", out.detach().clone()), ("loss", loss.detach().clone())]
+                + [("grad." + k, p.grad.clone()) for k, p in m.named_parameters()]
+                + [("param." + k, p.detach().clone()) for k, p in m.named_parameters()])
+
+    first, second = step(), step()
+    for (k, u), (_, v) in zip(first, second):
+        assert torch.equal(u, v), k
+
+
 def test_model_full_shape_properties():
     """BASELINE cfg2 shape (T=800, N=32, 4 x BiLSTM-512): oracle-free checks that do not depend on size."""
     from ctc_pytorch_b200.model import CTC_Model

@@ -1,6 +1,7 @@
 """CPU suite: pins the oracle (oracle/*.py) against (a) the committed golden vectors generated from the
-unmodified reference, (b) the reference itself when /root/reference is mounted (build container only),
-(c) torch's own CPU kernels, which is where the reference's arithmetic for the model and the loss lives."""
+unmodified reference, (b) what the reference itself returned on the inputs of the `*_reference_live` tests
+(tests/golden/reference_live.*, recorded by oracle/make_golden_live.py), (c) torch's own CPU kernels, which is where the
+reference's arithmetic for the model and the loss lives."""
 import json
 import os
 
@@ -9,9 +10,14 @@ import pytest
 import torch
 import torch.nn as nn
 
-from oracle import ctc_ref, decode_ref, model_ref, ref_shim
+from oracle import ctc_ref, decode_ref, model_ref
 
-HAVE_REF = ref_shim.available()
+
+@pytest.fixture(scope="module")
+def reference_live(golden_dir):
+    """(json, npz) of the reference's recorded answers."""
+    meta = json.load(open(os.path.join(golden_dir, "reference_live.json")))
+    return meta, np.load(os.path.join(golden_dir, "reference_live.npz"))
 
 
 # ---------------------------------------------------------------------------------------------- CTC
@@ -107,35 +113,32 @@ def test_lm_oracle_backoff(golden_dir):
         assert lm.bigram("a", "b") == lm.uni["a"][1] + lm.uni["b"][0]
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree only exists in the build container")
-def test_decode_oracle_matches_reference_live(golden_dir):
-    ref = ref_shim.load()
-    units = ["blank", "UNK", "a", "b", "c", "d", "e", "f"]
+def test_decode_oracle_matches_reference_live(golden_dir, reference_live):
+    """Bigram table, beam / greedy strings and wer / cer of the oracle equal what the reference's LanguageModel, BeamDecoder,
+    GreedyDecoder and Decoder returned on the same log-probs."""
+    meta, arrs = reference_live
+    rec = meta["decode"]
+    units = rec["units"]
     int2char = dict(enumerate(units))
-    arpa = os.path.join(golden_dir, "lm_c8.arpa")
-    lm = decode_ref.BigramLM(arpa)
-    rlm = ref.LanguageModel(arpa_file=arpa)
-    for w1 in units[1:] + [""]:
-        for w2 in units[1:] + [""]:
-            assert lm.bigram(w1, w2) == rlm.get_bi_prob(w1, w2)
-    for seed in range(6):
-        g = torch.Generator().manual_seed(100 + seed)
-        T, N, C = 24, 3, 8
-        logits = 2.5 * torch.randn(T, N, C, generator=g)
-        logits[:, :, 0] += 1.5
-        lp = torch.log_softmax(logits, -1)
-        lens = [T, T - 5, T // 2]
-        for width, alpha in ((2, 0.05), (8, 0.2)):
-            dec = ref.BeamDecoder(int2char, beam_width=width, blank_index=0, space_idx=-1, lm_path=arpa, lm_alpha=alpha)
-            want = dec.decode(lp, lens)
+    lm = decode_ref.BigramLM(os.path.join(golden_dir, rec["arpa"]))
+    words = rec["words"]
+    for i, w1 in enumerate(words):
+        for j, w2 in enumerate(words):
+            assert lm.bigram(w1, w2) == rec["bigram"][i][j]
+    assert len(rec["cases"]) == 6
+    for case in rec["cases"]:
+        lp = torch.from_numpy(arrs["decode/lp%d" % case["seed"]])
+        lens = case["lens"]
+        assert len(case["beams"]) == 2
+        for beam in case["beams"]:
             probs = torch.exp(lp.transpose(0, 1)).numpy()
-            _, got = decode_ref.beam_search(probs, lens, units, width, lm, alpha)
-            assert got == want
-        gd = ref.GreedyDecoder(int2char, space_idx=-1, blank_index=0)
-        assert decode_ref.greedy_strings(lp.numpy(), lens, int2char) == gd.decode(lp, lens)
-        d = ref.Decoder(int2char, space_idx=-1, blank_index=0)
-        assert d.cer(" a b c", " a c") == decode_ref.cer(" a b c", " a c")
-        assert d.wer("a b c d", "a c d e") == decode_ref.wer("a b c d", "a c d e")
+            _, got = decode_ref.beam_search(probs, lens, units, beam["beam_width"], lm, beam["lm_alpha"])
+            assert got == beam["strings"]
+        assert decode_ref.greedy_strings(lp.numpy(), lens, int2char) == case["greedy"]
+    a, b, want = rec["cer"]
+    assert decode_ref.cer(a, b) == want
+    a, b, want = rec["wer"]
+    assert decode_ref.wer(a, b) == want
 
 
 # ---------------------------------------------------------------------------------------------- model
@@ -172,20 +175,24 @@ def test_model_oracle_matches_golden(golden_dir, name):
         np.testing.assert_allclose(m(x).numpy(), g["out_eval"], atol=1e-6)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree only exists in the build container")
-def test_model_oracle_matches_reference_live():
-    from oracle.make_golden import MODEL_CASES, model_args
-    ref = ref_shim.load()
+def test_model_oracle_matches_reference_live(reference_live):
+    """The oracle, with the reference's weights (re-created from the seed, verified by checksum), gives the reference
+    CTC_Model's outputs in train mode and then in eval mode."""
+    from oracle.make_golden import MODEL_CASES
+    meta, arrs = reference_live
+    assert sorted(meta["model"]["checksum"]) == sorted(MODEL_CASES)
     for name, cfg in MODEL_CASES.items():
         torch.manual_seed(cfg["seed"])
-        rm = ref.CTC_Model(**model_args(cfg))
         om = _build_oracle(cfg)
-        om.load_state_dict(rm.state_dict())
+        want_sum = meta["model"]["checksum"][name]
+        assert list(om.state_dict()) == list(want_sum)
+        for k, v in om.state_dict().items():
+            assert abs(float(v.double().abs().sum()) - want_sum[k]) <= 1e-9 * max(1.0, want_sum[k]), (name, k)
         x, *_ = model_ref.synthetic_batch(cfg["T"], cfg["N"], cfg["F"], cfg["C"], cfg["S"], cfg["seed"])
+        assert np.array_equal(x.numpy(), arrs["model/%s/x" % name])
         for mode in ("train", "eval"):
-            getattr(rm, mode)()
             getattr(om, mode)()
-            a, b = rm(x), om(x)
+            a, b = torch.from_numpy(arrs["model/%s/%s" % (name, mode)]), om(x)
             # same library kernels, different reduction order inside BatchNorm -> float32 round-off only
             assert torch.allclose(a, b, atol=2e-6, rtol=0), (name, mode, (a - b).abs().max())
 
@@ -231,29 +238,36 @@ def test_packed_oracle_matches_golden(golden_dir):
         np.testing.assert_allclose(m(x, lens).numpy(), g["logp_eval"], atol=5e-6)
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/my_863_corpus/steps"), reason="reference tree only exists in the build container")
-def test_packed_oracle_matches_reference_live():
-    import sys
+def test_packed_oracle_matches_reference_live(reference_live):
+    """The packed oracle, with the unmodified 863 CTC_RNN's weights (re-created from the seed, verified by checksum), gives its
+    activations, loss and gradients (a fixed sample of 1024 entries per parameter, plus every gradient's norm)."""
     from oracle import packed_ref
-    sys.path.insert(0, "/root/reference/my_863_corpus/steps")
-    import model as m863
-    for seed, (T, N, H, L, bn) in enumerate([(18, 3, 128, 2, True), (25, 4, 128, 3, True), (12, 2, 128, 2, False)]):
+    from oracle.make_golden_live import PACKED_CASES, grad_sample_index
+    meta, arrs = reference_live
+    cases = meta["packed"]["cases"]
+    assert [(c["T"], c["N"], c["H"], c["L"], c["bn"]) for c in cases] == [tuple(c) for c in PACKED_CASES]
+    for case in cases:
+        seed, T, N, H, L, bn = case["seed"], case["T"], case["N"], case["H"], case["L"], case["bn"]
         torch.manual_seed(100 + seed)
-        ref = m863.CTC_RNN(rnn_input_size=40, rnn_hidden_size=H, rnn_layers=L, rnn_type=nn.LSTM, bidirectional=True,
-                           batch_norm=bn, num_class=9, drop_out=0.0)
         mine = packed_ref.RefPackedModel(40, H, L, bn, 9)
-        mine.load_state_dict(ref.state_dict())
+        assert list(mine.state_dict()) == list(case["checksum"])
+        for k, v in mine.state_dict().items():
+            assert abs(float(v.double().abs().sum()) - case["checksum"][k]) <= 1e-9 * max(1.0, case["checksum"][k]), k
         x, lens, tg, tsz = packed_ref.synthetic_packed_batch(T, N, 40, 9, 3, seed)
-        ref.train(); mine.train()
-        a = ref(nn.utils.rnn.pack_padded_sequence(x, lens))
+        mine.train()
+        a = torch.from_numpy(arrs["packed/%d/act" % seed])
         b = mine(x, lens)
         assert (a - b).abs().max().item() < 5e-6
-        la = packed_ref.warp_ctc_loss(a, tg, lens, tsz); la.backward()
+        la = case["loss"]
         lb = packed_ref.warp_ctc_loss(b, tg, lens, tsz); lb.backward()
-        assert abs(la.item() - lb.item()) < 1e-5 * abs(la.item())
-        pa, pb = dict(ref.named_parameters()), dict(mine.named_parameters())
-        for k in pa:
-            assert (pa[k].grad - pb[k].grad).abs().max().item() < 2e-5 * max(1.0, pa[k].grad.abs().max().item()), k
+        assert abs(la - lb.item()) < 1e-5 * abs(la)
+        for k, p in mine.named_parameters():
+            want, g = case["grads"][k], p.grad.reshape(-1)
+            tol = 2e-5 * max(1.0, want["maxabs"])
+            got = g[torch.from_numpy(grad_sample_index(g.numel(), k))]
+            assert (got - torch.from_numpy(arrs["packed/%d/grad/%s" % (seed, k)])).abs().max().item() < tol, k
+            assert abs(g.abs().max().item() - want["maxabs"]) < tol, k
+            assert abs(g.norm().item() - want["norm"]) < 1e-4 * max(1.0, want["norm"]), k
 
 
 # ------------------------------------------------------------------- host batch assembly (N2)
@@ -274,19 +288,16 @@ def test_batch_oracle_matches_golden(golden_dir):
         assert np.array_equal(tg, g["case%d/targets" % ci]) and np.array_equal(tsz, g["case%d/target_sizes" % ci])
 
 
-@pytest.mark.skipif(not os.path.isdir("/root/reference/timit/utils"), reason="reference tree only exists in the build container")
-def test_batch_oracle_matches_reference_live():
-    import sys
-    import types
+def test_batch_oracle_matches_reference_live(reference_live):
+    """Splicing and frame skipping of the oracle equal the reference's utils/tools.py make_context + skip_feat."""
     from oracle import batch_ref
-    sys.path.insert(0, "/root/reference/timit")
-    sys.path.insert(0, "/root/reference/timit/utils")
-    sys.modules.setdefault("kaldiio", types.ModuleType("kaldiio"))
-    import tools
+    meta, arrs = reference_live
+    assert meta["batch"]["cases"] == [[0, 0, 1], [4, 0, 1], [0, 3, 2], [2, 2, 5], [7, 7, 3]]
     rng = np.random.RandomState(3)
-    for left, right, skip in [(0, 0, 1), (4, 0, 1), (0, 3, 2), (2, 2, 5), (7, 7, 3)]:
+    for ci, (left, right, skip) in enumerate(meta["batch"]["cases"]):
         f = rng.randn(rng.randint(1, 30), 5).astype(np.float32)
-        a = tools.skip_feat(tools.make_context(f, left, right), skip)
+        assert np.array_equal(f, arrs["batch/%d/feat" % ci])
+        a = arrs["batch/%d/out" % ci]
         b = batch_ref.skipped(batch_ref.spliced(f, left, right), skip)
         assert a.shape == b.shape and np.array_equal(a, b)
 

@@ -1,7 +1,9 @@
 """CPU tests of the training-loop services (ctc_pytorch_b200/train.py): the lr / rollback schedule against the oracle's
-restatement of train_ctc.py:162-231 AND against the reference's own loop source exec'ed with stubs (oracle/train_live.py),
-and checkpoint interchange with the unmodified reference when it is mounted."""
-import random
+restatement of train_ctc.py:162-231 AND against what the reference's own loop source, exec'ed with stubs (oracle/train_live.py),
+produced, and checkpoint interchange with the unmodified reference's package layout (both recorded in
+tests/golden/reference_live.json by oracle/make_golden_live.py)."""
+import json
+import os
 
 import pytest
 import torch
@@ -9,30 +11,18 @@ import torch.nn as nn
 
 from ctc_pytorch_b200.model import CTC_Model
 from ctc_pytorch_b200.train import DevLossSchedule, load_package
-from oracle import ref_shim, train_ref
+from oracle import train_ref
+from oracle.make_golden_live import CHECKPOINT_RNN_PARAM as RNN_PARAM
 
-HAVE_REF = ref_shim.available()
 
-
-def _sequence(seed, n):
-    rng = random.Random(seed)
-    loss, out_l, out_a = 40.0 + rng.random() * 10, [], []
-    for i in range(n):
-        r = rng.random()
-        if r < 0.45:
-            loss -= rng.random() * 2.0          # clear improvement
-        elif r < 0.8:
-            loss += (rng.random() - 0.5) * 0.02  # plateau inside the +-end_adjust_acc band
-        else:
-            loss += rng.random() * 3.0          # divergence -> immediate halving
-        out_l.append(loss)
-        out_a.append(rng.random())
-    return out_l, out_a
+@pytest.fixture(scope="module")
+def reference_live(golden_dir):
+    return json.load(open(os.path.join(golden_dir, "reference_live.json")))
 
 
 @pytest.mark.parametrize("seed", range(12))
 def test_schedule_matches_reference_policy(seed):
-    losses, accs = _sequence(seed, 120)
+    losses, accs = train_ref.scripted_sequence(seed, 120)
     init_lr, decay, eps, epochs = 1e-3, 0.5, 0.05, 100
     want, final = train_ref.schedule_trace(losses, accs, init_lr, decay, eps, epochs)
     sched = DevLossSchedule(init_lr, decay, eps)
@@ -49,17 +39,20 @@ def test_schedule_matches_reference_policy(seed):
     assert any(w["rollback"] for w in want)   # the sequences do exercise the halving path
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference modules neither mounted nor staged")
 @pytest.mark.parametrize("seed", range(12))
-def test_schedule_pinned_to_the_reference_loop_source(seed):
+def test_schedule_pinned_to_the_reference_loop_source(seed, reference_live):
     """The policy's oracle is the reference's OWN statements: oracle/train_live.py cuts the `while not stop_train:` loop out of the
     unmodified steps/train_ctc.py (lines 159-231), execs it with stubs, and both the restatement (oracle/train_ref.py) and
     DevLossSchedule must reproduce its learning rates, roll-backs and final bookkeeping epoch by epoch."""
-    from oracle import train_live
-    losses, accs = _sequence(seed, 120)
-    losses[0] = 30.0           # below the initial loss_best = 1000 so that the counter is bound, as in any real run
+    rec = reference_live["schedule"]
+    trace = rec["traces"][seed]
+    assert trace["seed"] == seed
+    losses, accs = train_ref.scripted_sequence(seed, 120)
+    losses[0] = rec["first_loss"]   # below the initial loss_best = 1000 so that the counter is bound, as in any real run
     init_lr, decay, eps, epochs = 1e-3, 0.5, 0.05, 100
-    live, final = train_live.reference_schedule_trace(losses, accs, init_lr, decay, eps, epochs)
+    assert (rec["init_lr"], rec["decay"], rec["end_adjust_acc"], rec["num_epoches"]) == (init_lr, decay, eps, epochs)
+    live = [{"lr": lr, "rollback": rb} for lr, rb in zip(trace["lr"], trace["rollback"])]
+    final = trace["final"]
     restated, rfinal = train_ref.schedule_trace(losses, accs, init_lr, decay, eps, epochs)
     sched = DevLossSchedule(init_lr, decay, eps)
     ours, count = [], 0
@@ -86,10 +79,6 @@ def test_schedule_reproduces_the_unbound_counter_quirk():
         train_ref.schedule_trace([1000.0], [0.1], 1e-3, 0.5, 0.05, 5)
 
 
-RNN_PARAM = {"rnn_input_size": 40, "rnn_hidden_size": 128, "rnn_layers": 2, "rnn_type": nn.LSTM, "bidirectional": True,
-             "batch_norm": True}
-
-
 def test_package_roundtrip_cpu():
     m = CTC_Model(rnn_param=RNN_PARAM, num_class=11, drop_out=0.1)
     opt = torch.optim.Adam(m.parameters(), lr=1e-3)
@@ -101,19 +90,29 @@ def test_package_roundtrip_cpu():
         assert k1 == k2 and torch.equal(v1, v2)
 
 
-@pytest.mark.skipif(not HAVE_REF, reason="reference tree not mounted")
-def test_checkpoint_interchange_with_reference():
-    ref = ref_shim.load()
+def test_checkpoint_interchange_with_reference(reference_live):
+    """A package of ours has the reference's layout (keys, constructor fields, state_dict names and shapes, so the reference's
+    constructor + load_state_dict accept it), and a package in the reference's layout, holding the reference's weights
+    (re-created from the seed, verified by checksum), loads into ours unchanged."""
+    rec = reference_live["checkpoint"]
     ours = CTC_Model(rnn_param=RNN_PARAM, num_class=11, drop_out=0.1)
-    theirs = ref.CTC_Model(rnn_param=RNN_PARAM, num_class=11, drop_out=0.1)
     # ours -> reference (test_ctc.py:37-60 style)
     pkg = CTC_Model.save_package(ours, epoch={"epoch": 1})
-    rebuilt = ref.CTC_Model(rnn_param=pkg["rnn_param"], add_cnn=pkg["add_cnn"], cnn_param=pkg["cnn_param"],
-                            num_class=pkg["num_class"], drop_out=pkg["_drop_out"])
-    rebuilt.load_state_dict(pkg["state_dict"])
+    assert sorted(pkg.keys()) == rec["keys"]
+    for k, v in rec["fields"].items():
+        got = pkg[k]
+        if k == "rnn_param":
+            got = dict(got, rnn_type=got["rnn_type"].__name__)
+        assert got == v, k
+    assert [[k, list(v.shape)] for k, v in pkg["state_dict"].items()] == rec["state_dict"]
     # reference -> ours
-    rpkg = ref.CTC_Model.save_package(theirs, epoch={"epoch": 1})
-    assert set(rpkg.keys()) == set(pkg.keys())
+    torch.manual_seed(rec["seed"])
+    sd = CTC_Model(rnn_param=RNN_PARAM, num_class=11, drop_out=0.1).state_dict()
+    for k, v in sd.items():
+        assert abs(float(v.double().abs().sum()) - rec["checksum"][k]) <= 1e-9 * max(1.0, rec["checksum"][k]), k
+    rpkg = dict(rec["fields"], state_dict=sd)
+    rpkg["rnn_param"] = dict(rpkg["rnn_param"], rnn_type=getattr(nn, rpkg["rnn_param"]["rnn_type"]))
     m2, _ = load_package(rpkg, device="cpu")
-    for (k1, v1), (k2, v2) in zip(theirs.state_dict().items(), m2.state_dict().items()):
+    assert list(m2.state_dict()) == list(sd)
+    for (k1, v1), (k2, v2) in zip(sd.items(), m2.state_dict().items()):
         assert k1 == k2 and torch.equal(v1, v2)
