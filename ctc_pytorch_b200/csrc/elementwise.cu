@@ -74,6 +74,58 @@ __global__ void pack_lstm_weights_kernel(const float* __restrict__ wih_f, const 
     }
 }
 
+// torch row of packed gate row p of a layer run at Hp >= H units (units >= H are zero padding), or -1 for a zero row
+__device__ __forceinline__ int padded_src_row(int p, int H, int Hp, int gates) {
+    const int orow = packed_to_orig_row(p, Hp), q = orow / Hp, u = orow % Hp;
+    return (u < H && q < gates) ? q * H + u : -1;
+}
+// torch input column of device input column i: blocks of i_blk real columns spread i_blk_p apart (-1: zero padding)
+__device__ __forceinline__ int padded_src_col(int i, int i_blk, int i_blk_p) {
+    const int off = i % i_blk_p;
+    return off < i_blk ? (i / i_blk_p) * i_blk + off : -1;
+}
+
+// The same operand layouts as pack_lstm_weights_kernel for a layer run at Hp = 128 * ceil(H / 128) units: the Hp - H extra units
+// get zero rows in every matrix and zero columns in the recurrent ones, and the input columns are spread the way the layer below
+// leaves its output (I_dev = (I / i_blk) * i_blk_p device columns). Those units then stay exactly zero (DESIGN.md §3.2).
+__global__ void pack_lstm_weights_padded_kernel(const float* __restrict__ wih_f, const float* __restrict__ whh_f,
+                                                const float* __restrict__ wih_r, const float* __restrict__ whh_r,
+                                                __nv_bfloat16* __restrict__ wih_p, __nv_bfloat16* __restrict__ wihT_p,
+                                                __nv_bfloat16* __restrict__ whh_p, __nv_bfloat16* __restrict__ whhT_p, int H,
+                                                int Hp, int I, int i_blk, int i_blk_p, int I_dev, int Ipad, int part, int gates) {
+    const long long tid = static_cast<long long>(blockIdx.x) * blockDim.x + threadIdx.x;
+    const long long stride = static_cast<long long>(gridDim.x) * blockDim.x;
+    const int G4 = 4 * Hp, G8 = 8 * Hp;
+    // wih_p [8Hp, Ipad]
+    for (long long e = tid; e < static_cast<long long>(G8) * Ipad; e += stride) {
+        const int R = static_cast<int>(e / Ipad), i = static_cast<int>(e % Ipad);
+        const int orow = padded_src_row(R % G4, H, Hp, gates), ic = i < I_dev ? padded_src_col(i, i_blk, i_blk_p) : -1;
+        const float* w = R >= G4 ? wih_r : wih_f;
+        wih_p[e] = bf16_part((orow >= 0 && ic >= 0) ? w[static_cast<size_t>(orow) * I + ic] : 0.0f, part);
+    }
+    // wihT_p [I_dev, 8Hp]
+    for (long long e = tid; e < static_cast<long long>(I_dev) * G8; e += stride) {
+        const int i = static_cast<int>(e / G8), R = static_cast<int>(e % G8);
+        const int orow = padded_src_row(R % G4, H, Hp, gates), ic = padded_src_col(i, i_blk, i_blk_p);
+        const float* w = R >= G4 ? wih_r : wih_f;
+        wihT_p[e] = bf16_part((orow >= 0 && ic >= 0) ? w[static_cast<size_t>(orow) * I + ic] : 0.0f, part);
+    }
+    // whh_p [8Hp, Hp]
+    for (long long e = tid; e < static_cast<long long>(G8) * Hp; e += stride) {
+        const int R = static_cast<int>(e / Hp), k = static_cast<int>(e % Hp);
+        const int orow = padded_src_row(R % G4, H, Hp, gates);
+        const float* w = R >= G4 ? whh_r : whh_f;
+        whh_p[e] = bf16_part((orow >= 0 && k < H) ? w[static_cast<size_t>(orow) * H + k] : 0.0f, part);
+    }
+    // whhT_p [(dir,q,m), k] = whh_dir[q*H + k][m]
+    for (long long e = tid; e < static_cast<long long>(G8) * Hp; e += stride) {
+        const int R = static_cast<int>(e / Hp), k = static_cast<int>(e % Hp);
+        const int q = (R % G4) / Hp, m = R % Hp;
+        const float* w = R >= G4 ? whh_r : whh_f;
+        whhT_p[e] = bf16_part((q < gates && k < H && m < H) ? w[(static_cast<size_t>(q) * H + k) * H + m] : 0.0f, part);
+    }
+}
+
 // src element (r, c) lives at src[(r / n_inner) * s_outer + (r % n_inner) * s_inner + c].
 __global__ void __launch_bounds__(256)
 cast_transpose_kernel(const float* __restrict__ src, long long s_outer, long long s_inner, int n_inner,
@@ -502,6 +554,26 @@ extern "C" CTCB200_API int ctcb200_pack_lstm_weights(const float* wih_f, const f
     pack_lstm_weights_kernel<<<stream_grid(work, 1024), 256, 0, stream>>>(
         wih_f, whh_f, wih_r, whh_r, static_cast<__nv_bfloat16*>(wih_p), static_cast<__nv_bfloat16*>(wihT_p),
         static_cast<__nv_bfloat16*>(whh_p), static_cast<__nv_bfloat16*>(whhT_p), H, I, Ipad, part, gates);
+    CTCB_LAUNCH_CHECK();
+    return OK;
+}
+
+extern "C" CTCB200_API int ctcb200_pack_lstm_weights_padded(const float* wih_f, const float* whh_f, const float* wih_r,
+                                                            const float* whh_r, void* wih_p, void* wihT_p, void* whh_p,
+                                                            void* whhT_p, int H, int Hp, int I, int i_blk, int i_blk_p, int Ipad,
+                                                            int part, int gates, ctcb200_stream_t stream_) {
+    cudaStream_t stream = static_cast<cudaStream_t>(stream_);
+    CTCB_REQUIRE(H >= 1 && Hp >= H && Hp % 32 == 0, "pack_lstm_weights_padded: bad hidden sizes H=%d Hp=%d", H, Hp);
+    CTCB_REQUIRE(I > 0 && i_blk >= 1 && i_blk_p >= i_blk && I % i_blk == 0,
+                 "pack_lstm_weights_padded: bad input map I=%d i_blk=%d i_blk_p=%d", I, i_blk, i_blk_p);
+    const int I_dev = (I / i_blk) * i_blk_p;
+    CTCB_REQUIRE(Ipad >= I_dev && Ipad % 8 == 0, "pack_lstm_weights_padded: Ipad=%d below the %d device columns", Ipad, I_dev);
+    CTCB_REQUIRE(gates == 4 || gates == 3 || gates == 1, "pack_lstm_weights_padded: gates %d not in {4 LSTM, 3 GRU, 1 RNN}", gates);
+    const long long work = static_cast<long long>(8) * Hp * (Ipad > Hp ? Ipad : Hp);
+    pack_lstm_weights_padded_kernel<<<stream_grid(work, 1024), 256, 0, stream>>>(
+        wih_f, whh_f, wih_r, whh_r, static_cast<__nv_bfloat16*>(wih_p), static_cast<__nv_bfloat16*>(wihT_p),
+        static_cast<__nv_bfloat16*>(whh_p), static_cast<__nv_bfloat16*>(whhT_p), H, Hp, I, i_blk, i_blk_p, I_dev, Ipad, part,
+        gates);
     CTCB_LAUNCH_CHECK();
     return OK;
 }

@@ -194,6 +194,12 @@ enum { CELL_LSTM = 0, CELL_GRU = 1, CELL_RNN = 2 };
 // per operand image: with their short chain the extra waits cost more than the overlap returns (measured: BPTT 1.48 -> 1.7).
 // ------------------------------------------------------------------------------------------------
 constexpr int MAX_KB = 8;   // K blocks of 64 units in a one-cluster kernel (H <= 512)
+// K elements of a [128 x H] weight slice that fit tensor memory next to the accumulators: columns [64, 64 + 896/2) of 512. The
+// bf16 global-exchange kernels (EX = 0) take H up to 1024; the K blocks past 896 sit in shared memory (TMA, SWIZZLE_128B) and
+// go through the SS-form MMA, as the x3 kernels' W_lo slice does.
+constexpr int TMEM_K_MAX = 896;
+constexpr int MAX_HIDDEN = 1024;     // largest (device) hidden size of the recurrent kernels
+constexpr int MAX_HIDDEN_X3 = 640;   // split-operand mode: the W_lo slice and the hi/lo operand image must fit shared memory
 __device__ __forceinline__ uint32_t exchange_peer(int me, int pos, int ctas) {   // pos-th destination of CTA `me`
     const int pairs = ctas >> 1;
     int c = (me >> 1) + (pos >> 1);
@@ -301,8 +307,11 @@ lstm_fwd_kernel(const __grid_constant__ CUtensorMap tmWlo, FwdParams p) {
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int H = p.H, T = p.T, N = p.N;
     const int himg_bytes = H * NB * 2 * PARTS;
-    uint8_t* sW = smem;                                              // X3: the W_lo slice [128 x H] bf16
-    uint8_t* sH = sW + (X3 ? 128 * H * 2 : 0);                       // BULK: two parities, else one buffer
+    constexpr bool SPILL = EX == 0 && !X3;                           // H > TMEM_K_MAX possible (see TMEM_K_MAX)
+    const int k_tmem = (SPILL && H > TMEM_K_MAX) ? TMEM_K_MAX : H;   // K elements of the W slice resident in TMEM
+    const int kb_tmem = k_tmem / 64;
+    uint8_t* sW = smem;                                              // X3: the W_lo slice [128 x H] bf16; SPILL: K >= k_tmem
+    uint8_t* sH = sW + (X3 ? 128 * H * 2 : (SPILL ? 128 * (H - k_tmem) * 2 : 0));   // BULK: two parities, else one buffer
     float* sS = reinterpret_cast<float*>(sH + (BULK ? 2 : 1) * himg_bytes);
     uint4* sOut = reinterpret_cast<uint4*>(sS + 32 * S_STRIDE);      // BULK only: staging of this CTA's block [hi | lo]
     uint64_t* bars = reinterpret_cast<uint64_t*>(sOut + (BULK ? PARTS * OUT_CHUNKS : 0));
@@ -331,9 +340,9 @@ lstm_fwd_kernel(const __grid_constant__ CUtensorMap tmWlo, FwdParams p) {
             for (int i = 0; i < 2 * HB_STRIDE; ++i) mbar_expect_tx(&h_full[i], (KBB ? 2 : ctas) * BLK_STRIDE);
         }
     }
-    // TMEM: up to four accumulators in columns [0, 64), the W_hi slice (A operand) in columns [64, 64 + H/2)
+    // TMEM: up to four accumulators in columns [0, 64), the W_hi slice (A operand) in columns [64, 64 + k_tmem/2)
     uint32_t tmem_cols = 64;
-    while (tmem_cols < 64u + H / 2) tmem_cols <<= 1;
+    while (tmem_cols < 64u + k_tmem / 2) tmem_cols <<= 1;
     if (warp == 1) tmem_alloc(tmem_slot, tmem_cols);
     if constexpr (BULK) {
         // h_{-1} = 0: the first operand buffer starts zeroed
@@ -346,11 +355,20 @@ lstm_fwd_kernel(const __grid_constant__ CUtensorMap tmWlo, FwdParams p) {
     const uint32_t tmem_base = *tmem_slot;
     if constexpr (CL) cluster_sync_all();  // peers' barriers are initialised before anyone arrives on them
 
-    if (warp < 4) load_weights_to_tmem(p.w + (static_cast<size_t>(dir) * 4 * H + j * 128) * H, H, tmem_base, 64, warp, lane);
+    if (warp < 4)
+        load_weights_to_tmem(p.w + (static_cast<size_t>(dir) * 4 * H + j * 128) * H, k_tmem, tmem_base, 64, warp, lane,
+                             SPILL ? H : 0);
     if constexpr (X3) {
         if (tid == 0) {
             mbar_expect_tx(w_full, 128 * H * 2);
             for (int kb = 0; kb < kblocks; ++kb) tma_load_2d(sW + kb * 16384, &tmWlo, w_full, kb * 64, dir * 4 * H + j * 128);
+        }
+    }
+    if constexpr (SPILL) {   // (tmWlo maps the W_hi image here)
+        if (tid == 0 && k_tmem < H) {
+            mbar_expect_tx(w_full, 128 * (H - k_tmem) * 2);
+            for (int kb = kb_tmem; kb < kblocks; ++kb)
+                tma_load_2d(sW + (kb - kb_tmem) * 16384, &tmWlo, w_full, kb * 64, dir * 4 * H + j * 128);
         }
     }
     tc_fence_before();
@@ -407,6 +425,7 @@ lstm_fwd_kernel(const __grid_constant__ CUtensorMap tmWlo, FwdParams p) {
         // arithmetic so the descriptors live in uniform registers, one elected lane issues each tcgen05.mma
         if (warp < p.mma_split) {
             if constexpr (X3) { if (t == 0) mbar_wait(w_full, 0); }
+            if constexpr (SPILL) { if (t == 0 && k_tmem < H) mbar_wait(w_full, 0); }
             if constexpr (KBB) {
                 // per-K-block waits inside the loop; the issuing warps took part in last step's CTA barriers themselves
             } else if constexpr (BULK) {
@@ -438,7 +457,15 @@ lstm_fwd_kernel(const __grid_constant__ CUtensorMap tmWlo, FwdParams p) {
                 // 64 K elements = two SWIZZLE_64B blocks of the B image, two K=16 slices (32 bytes apart) in each
                 const uint64_t bd = umma_desc_sw64(b0 + kb * (2 * BLK_STRIDE));
                 const uint32_t ta = tmem_base + 64 + kb * 32;
-                if (leader) {
+                if (SPILL && kb >= kb_tmem) {   // this K block of W sits in shared memory
+                    const uint64_t ad = umma_desc_sw128(a0 + (kb - kb_tmem) * 16384);
+                    if (leader) {
+                        umma_bf16(dacc, ad, bd, idesc, it != kfirst ? 1u : 0u);
+                        umma_bf16(dacc, ad + 2, bd + 2, idesc, 1u);
+                        umma_bf16(dacc, ad + 4, bd + B2, idesc, 1u);
+                        umma_bf16(dacc, ad + 6, bd + B2 + 2, idesc, 1u);
+                    }
+                } else if (leader) {
                     umma_bf16_ts(dacc, ta, bd, idesc, it != kfirst ? 1u : 0u);
                     umma_bf16_ts(dacc, ta + 8, bd + 2, idesc, 1u);
                     umma_bf16_ts(dacc, ta + 16, bd + B2, idesc, 1u);
@@ -933,8 +960,11 @@ lstm_bwd_kernel(const __grid_constant__ CUtensorMap tmWTlo, BwdParams p) {
     uint8_t* smem = reinterpret_cast<uint8_t*>((reinterpret_cast<uintptr_t>(smem_raw) + 1023) & ~uintptr_t(1023));
     const int H = p.H, T = p.T, N = p.N;
     const int img_bytes = H * NB * 2 * PARTS;
-    uint8_t* sW = smem;                                               // X3: the W^T_lo slice [128 x H] bf16
-    uint8_t* sB = sW + (X3 ? 128 * H * 2 : 0);                        // BULK: two parities, else one buffer
+    constexpr bool SPILL = EX == 0 && !X3;                            // H > TMEM_K_MAX possible (see TMEM_K_MAX)
+    const int k_tmem = (SPILL && H > TMEM_K_MAX) ? TMEM_K_MAX : H;    // K elements of the W^T slice resident in TMEM
+    const int kb_tmem = k_tmem / 64;
+    uint8_t* sW = smem;                                               // X3: the W^T_lo slice [128 x H] bf16; SPILL: K >= k_tmem
+    uint8_t* sB = sW + (X3 ? 128 * H * 2 : (SPILL ? 128 * (H - k_tmem) * 2 : 0));   // BULK: two parities, else one buffer
     float* sR = reinterpret_cast<float*>(sB + (BULK ? 2 : 1) * img_bytes);  // [4 src][NB][32] partial dh blocks
     uint4* sOut = reinterpret_cast<uint4*>(sR + 4 * NB * 32);         // BULK only: [4 gates][PARTS][OUT_CHUNKS]
     float* sP = reinterpret_cast<float*>(sOut + (BULK ? 4 * PARTS * OUT_CHUNKS : 0));  // BULK only: [4 dst][NB][32] partial staging
@@ -972,7 +1002,7 @@ lstm_bwd_kernel(const __grid_constant__ CUtensorMap tmWTlo, BwdParams p) {
         }
     }
     uint32_t tmem_cols = 64;
-    while (tmem_cols < 64u + H / 2) tmem_cols <<= 1;
+    while (tmem_cols < 64u + k_tmem / 2) tmem_cols <<= 1;
     if (warp == 1) tmem_alloc(tmem_slot, tmem_cols);
     if constexpr (BULK) {
         for (int i = tid; i < img_bytes / 16; i += LSTM_THREADS) reinterpret_cast<uint4*>(sB)[i] = make_uint4(0u, 0u, 0u, 0u);
@@ -986,12 +1016,20 @@ lstm_bwd_kernel(const __grid_constant__ CUtensorMap tmWTlo, BwdParams p) {
 
     // rows of the transposed gate block: (dir, q, unit); this CTA takes units [128 mb, +128)
     if (warp < 4)
-        load_weights_to_tmem(p.w + (static_cast<size_t>(dir * 4 + q) * H + mb * 128) * H, H, tmem_base, 64, warp, lane);
+        load_weights_to_tmem(p.w + (static_cast<size_t>(dir * 4 + q) * H + mb * 128) * H, k_tmem, tmem_base, 64, warp, lane,
+                             SPILL ? H : 0);
     if constexpr (X3) {
         if (tid == 0) {
             mbar_expect_tx(w_full, 128 * H * 2);
             for (int kb = 0; kb < kblocks; ++kb)
                 tma_load_2d(sW + kb * 16384, &tmWTlo, w_full, kb * 64, (dir * 4 + q) * H + mb * 128);
+        }
+    }
+    if constexpr (SPILL) {   // (tmWTlo maps the W^T_hi image here)
+        if (tid == 0 && k_tmem < H) {
+            mbar_expect_tx(w_full, 128 * (H - k_tmem) * 2);
+            for (int kb = kb_tmem; kb < kblocks; ++kb)
+                tma_load_2d(sW + (kb - kb_tmem) * 16384, &tmWTlo, w_full, kb * 64, (dir * 4 + q) * H + mb * 128);
         }
     }
     tc_fence_before();
@@ -1058,6 +1096,7 @@ lstm_bwd_kernel(const __grid_constant__ CUtensorMap tmWTlo, BwdParams p) {
         // (4) partial dh[128 units, NB] = W_q^T slice * dG_q (issued like the forward kernel's chain)
         if (warp < p.mma_split) {
             if constexpr (X3) { if (t == 0) mbar_wait(w_full, 0); }
+            if constexpr (SPILL) { if (t == 0 && k_tmem < H) mbar_wait(w_full, 0); }
             if constexpr (KBB) {
                 // per-K-block waits inside the loop; the issuing warps took part in last step's CTA barriers themselves
             } else if constexpr (BULK) {
@@ -1088,7 +1127,15 @@ lstm_bwd_kernel(const __grid_constant__ CUtensorMap tmWTlo, BwdParams p) {
                 // 64 K elements = two SWIZZLE_64B blocks of the B image, two K=16 slices (32 bytes apart) in each
                 const uint64_t bd = umma_desc_sw64(b0 + kb * (2 * BLK_STRIDE));
                 const uint32_t ta = tmem_base + 64 + kb * 32;
-                if (leader) {
+                if (SPILL && kb >= kb_tmem) {   // this K block of W^T sits in shared memory
+                    const uint64_t ad = umma_desc_sw128(a0 + (kb - kb_tmem) * 16384);
+                    if (leader) {
+                        umma_bf16(dacc, ad, bd, idesc, it != kfirst ? 1u : 0u);
+                        umma_bf16(dacc, ad + 2, bd + 2, idesc, 1u);
+                        umma_bf16(dacc, ad + 4, bd + B2, idesc, 1u);
+                        umma_bf16(dacc, ad + 6, bd + B2 + 2, idesc, 1u);
+                    }
+                } else if (leader) {
                     umma_bf16_ts(dacc, ta, bd, idesc, it != kfirst ? 1u : 0u);
                     umma_bf16_ts(dacc, ta + 8, bd + 2, idesc, 1u);
                     umma_bf16_ts(dacc, ta + 16, bd + B2, idesc, 1u);
@@ -1814,6 +1861,7 @@ size_t lstm_smem_bytes(int NB, int H, bool bwd, int ex, bool x3) {
     const bool bulk = ex == 3;
     const size_t parts = x3 ? 2 : 1;
     size_t b = (x3 ? static_cast<size_t>(128) * H * 2 : 0) + static_cast<size_t>(bulk ? 2 : 1) * H * NB * 2 * parts;
+    if (!x3 && ex == 0 && H > TMEM_K_MAX) b += static_cast<size_t>(128) * (H - TMEM_K_MAX) * 2;   // W K blocks past TMEM
     if (bwd) b += static_cast<size_t>(4) * NB * 32 * 4 + (bulk ? static_cast<size_t>(4) * parts * NB * 4 * 16 + static_cast<size_t>(4) * NB * 32 * 4 : 0);
     else b += static_cast<size_t>(32) * (NB * 4 + 4) * 4 + (bulk ? parts * NB * 4 * 16 : 0);
     return exclusive_smem(b + 256 + 1024);
@@ -2065,7 +2113,7 @@ extern "C" CTCB200_API int64_t ctcb200_lstm_scratch_bytes(int N, int H) {
 
 extern "C" CTCB200_API int ctcb200_lstm_bwd_ctas(int N, int H, int batch_tile) {
     // SMs the (first) BPTT launch occupies: one CTA per SM, 4 gates x H/128 unit blocks x 2 directions x batch groups
-    if (H % 128 != 0 || H < 128 || H > 640 || N <= 0) return 0;
+    if (H % 128 != 0 || H < 128 || H > MAX_HIDDEN || N <= 0) return 0;
     const int nb = two_tile_path(H) ? 16 : pick_nb(N, H, batch_tile, true, exchange_mode(H) != 0);
     const int groups = (N + nb - 1) / nb;
     const int per_group = two_tile_path(H) ? 2 * 2 * (H / 128) : 2 * 4 * (H / 128);
@@ -2090,7 +2138,8 @@ int lstm_fwd_impl(const float* gx, const void* whh_packed, const void* whh_lo_pa
     const int cell_k = cell == 0 ? CELL_LSTM : (cell == 1 ? CELL_GRU : CELL_RNN);
     const bool plain = cell_k == CELL_LSTM;   // the pipelined / two-tile fast paths exist for the LSTM cell only
     CTCB_REQUIRE(T > 0 && N > 0, "lstm_fwd: empty T=%d N=%d", T, N);
-    CTCB_REQUIRE(H % 128 == 0 && H >= 128 && H <= 640, "lstm_fwd: hidden size %d must be a multiple of 128 in [128,640]", H);
+    CTCB_REQUIRE(H % 128 == 0 && H >= 128 && H <= (x3 ? MAX_HIDDEN_X3 : MAX_HIDDEN),
+                 "lstm_fwd: hidden size %d must be a multiple of 128 in [128,%d]", H, x3 ? MAX_HIDDEN_X3 : MAX_HIDDEN);
     FwdParams p;
     p.gx = gx; p.hout = hout; p.c_save = c_save;
     p.gates_save = x3 ? nullptr : static_cast<uint2*>(gates_save);
@@ -2258,7 +2307,8 @@ int lstm_bwd_impl(const float* dhout, const void* whhT_packed, const void* whhT_
     CTCB_REQUIRE(T > 0 && N > 0, "lstm_bwd: empty T=%d N=%d", T, N);
     CTCB_REQUIRE((reinterpret_cast<uintptr_t>(resident_counter) & 3) == 0, "lstm_bwd: resident_counter must be 4-byte aligned");
     CTCB_REQUIRE((bn_x == nullptr) == (bn_coef == nullptr), "lstm_bwd: bn_x and bn_coef must be given together");
-    CTCB_REQUIRE(H % 128 == 0 && H >= 128 && H <= 640, "lstm_bwd: hidden size %d must be a multiple of 128 in [128,640]", H);
+    CTCB_REQUIRE(H % 128 == 0 && H >= 128 && H <= (x3 ? MAX_HIDDEN_X3 : MAX_HIDDEN),
+                 "lstm_bwd: hidden size %d must be a multiple of 128 in [128,%d]", H, x3 ? MAX_HIDDEN_X3 : MAX_HIDDEN);
     CTCB_REQUIRE(plan_only || !x3 || dg_lo != nullptr, "lstm_bwd: the split-operand mode needs dg_lo");
     CTCB_REQUIRE((reinterpret_cast<uintptr_t>(progress_counter) & 3) == 0, "lstm_bwd: progress_counter must be 4-byte aligned");
     CTCB_REQUIRE(progress_counter == nullptr || chunk_T >= 1, "lstm_bwd: streamed gate gradients need chunk_T >= 1 (got %d)", chunk_T);

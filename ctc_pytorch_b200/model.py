@@ -137,6 +137,52 @@ def _gate_row_perm(H, dev):
     return _GATE_PERM[key]
 
 
+# ----------------------------------------------------------------------------------------------------
+# hidden sizes that are not a multiple of 128: every layer runs at Hp = 128 * ceil(H / 128) device units, the Hp - H extra units
+# carry zero weights and stay exactly zero (DESIGN.md §3.2). Torch shapes (parameters, gradients, state_dict) keep H; activation
+# and gradient buffers use the device layout, where the D*H real features of a layer output sit at columns d*Hp + unit.
+# ----------------------------------------------------------------------------------------------------
+MAX_HIDDEN = 1024        # largest device hidden size of the recurrent kernels
+MAX_HIDDEN_X3 = 640      # ... in the split-operand mode (its W_lo slice and hi/lo operand image must fit shared memory)
+
+
+def device_hidden(H):
+    """Device hidden size the recurrent kernels run a layer of torch hidden size H at."""
+    return _round_up(H, 128)
+
+
+def check_hidden(H, x3):
+    """Hidden sizes the recurrent kernels can run: a RuntimeError before anything is launched otherwise."""
+    if H < 1:
+        raise RuntimeError("rnn_hidden_size must be >= 1 (got %d)" % H)
+    Hp = device_hidden(H)
+    if Hp > MAX_HIDDEN:
+        raise RuntimeError("rnn_hidden_size %d is not supported: the recurrent kernels run hidden sizes up to %d"
+                           % (H, MAX_HIDDEN))
+    if x3 and Hp > MAX_HIDDEN_X3:
+        raise RuntimeError("precision='x3' runs hidden sizes up to %d (rnn_hidden_size %d runs at %d device units); use "
+                           "precision='bf16' for larger layers" % (MAX_HIDDEN_X3, H, Hp))
+    return Hp
+
+
+_UNIT_COLS = {}
+
+
+def unit_cols(H, Hp, D, dev):
+    """Device column of every torch feature of a [*, D*H] layer output in the padded [*, D*Hp] layout: d*Hp + unit."""
+    key = (H, Hp, D, str(dev))
+    if key not in _UNIT_COLS:
+        _UNIT_COLS[key] = (torch.arange(D, device=dev).view(D, 1) * Hp + torch.arange(H, device=dev)).reshape(-1)
+    return _UNIT_COLS[key]
+
+
+def pad_cols(w, cols, width):
+    """fp32 copy of w [..., D*H] with its columns scattered to `cols` of a zero [..., width] tensor."""
+    out = torch.zeros(w.shape[:-1] + (width,), dtype=torch.float32, device=w.device)
+    out.index_copy_(w.dim() - 1, cols, w.detach().float())
+    return out
+
+
 def _cast_t(src, s_outer, s_inner, n_inner, R, C, scale=None, shift=None, want=True, want_t=False, x3=False):
     """fp32 (strided rows) -> bf16 [R, Cp] and/or bf16 [C, (R/n_inner)*n_pad] with the batch axis padded to 8; returns
     (_Opnd or None, _Opnd or None). x3: every output also gets its remainder part."""
@@ -377,18 +423,29 @@ def _realign(src, lengths, T, N, W, split, direction, dst=None, accumulate=False
 
 
 class _BNState(object):
-    __slots__ = ("mean", "rstd", "scale", "shift", "batch")
+    __slots__ = ("mean", "rstd", "scale", "shift", "batch", "gamma", "cols")
 
 
-def _bn_prepare(bn, x2d, R, C, training, n_valid=0):
+def _bn_prepare(bn, x2d, R, C, training, n_valid=0, cols=None):
     """Statistics (training) or running-stat affine (eval) for BatchNorm1d `bn` over rows of x2d [R, C]. n_valid > 0: packed
-    mode, the statistics are over that many valid rows (the padding rows of x2d are zero)."""
+    mode, the statistics are over that many valid rows (the padding rows of x2d are zero). cols: device column of every torch
+    feature (padded hidden size, see unit_cols): the kernels then see a [C] parameter image with gamma = beta = 0 on the padding
+    columns, so scale = shift = 0 there, and only the torch buffers' own columns of the running statistics are updated."""
     dev = x2d.device
     st = _BNState()
     st.scale = torch.empty(C, dtype=torch.float32, device=dev)
     st.shift = torch.empty(C, dtype=torch.float32, device=dev)
+    st.cols = cols
     gamma = bn.weight if bn.affine else None
     beta = bn.bias if bn.affine else None
+    run_mean, run_var = bn.running_mean, bn.running_var
+    if cols is not None:
+        Cr = cols.numel()
+        gamma = pad_cols(gamma if gamma is not None else torch.ones(Cr, device=dev), cols, C)
+        beta = pad_cols(beta if beta is not None else torch.zeros(Cr, device=dev), cols, C)
+        if run_mean is not None:
+            run_mean, run_var = pad_cols(run_mean, cols, C), pad_cols(run_var, cols, C)
+    st.gamma = gamma if cols is not None else bn.weight
     use_batch = training or not bn.track_running_stats
     st.batch = use_batch
     if use_batch:
@@ -402,21 +459,27 @@ def _bn_prepare(bn, x2d, R, C, training, n_valid=0):
             if bn.momentum is None:
                 mom = 1.0 / float(bn.num_batches_tracked.item())
         _call("ctcb200_bn_train_stats", _lib.ptr(x2d), R, C, _lib.ptr(gamma), _lib.ptr(beta),
-              _lib.ptr(bn.running_mean if upd else None), _lib.ptr(bn.running_var if upd else None), mom,
+              _lib.ptr(run_mean if upd else None), _lib.ptr(run_var if upd else None), mom,
               float(bn.eps), _lib.ptr(st.mean), _lib.ptr(st.rstd), _lib.ptr(st.scale), _lib.ptr(st.shift),
               _lib.ptr(ws), int(n_valid), _lib.stream())
+        if upd and cols is not None:
+            bn.running_mean.copy_(run_mean.index_select(0, cols))
+            bn.running_var.copy_(run_var.index_select(0, cols))
     else:
         # frozen statistics (eval mode): the same per-column affine; mean / rstd kept for a possible backward pass
-        st.mean = bn.running_mean.detach().float().contiguous()
-        st.rstd = torch.rsqrt(bn.running_var.detach().float() + float(bn.eps)).contiguous()
-        _call("ctcb200_bn_eval_affine", _lib.ptr(gamma), _lib.ptr(beta), _lib.ptr(bn.running_mean),
-              _lib.ptr(bn.running_var), float(bn.eps), _lib.ptr(st.scale), _lib.ptr(st.shift), C, _lib.stream())
+        st.mean = run_mean.detach().float().contiguous()
+        st.rstd = torch.rsqrt(run_var.detach().float() + float(bn.eps)).contiguous()
+        _call("ctcb200_bn_eval_affine", _lib.ptr(gamma), _lib.ptr(beta), _lib.ptr(run_mean),
+              _lib.ptr(run_var), float(bn.eps), _lib.ptr(st.scale), _lib.ptr(st.shift), C, _lib.stream())
     return st
 
 
-def _packed_weights(model, li, rnn, H, I, Ipad, x3, dev):
+def _packed_weights(model, li, rnn, H, I, Ipad, x3, dev, Hp=None, Ir=None, i_blk=None):
     """bf16 operand layouts of one layer's four weight matrices (hi, and lo in x3 mode). Re-packed only when a parameter
-    changed since the last call (inference / evaluation loops reuse them; an optimizer step bumps the version counters)."""
+    changed since the last call (inference / evaluation loops reuse them; an optimizer step bumps the version counters).
+    Padded hidden size (Hp > H): the layouts are built at Hp from the torch-shaped weights (ctcb200_pack_lstm_weights_padded);
+    I is then the device input width, Ir the torch one, and the input columns come in blocks of i_blk spread Hp apart above
+    the first layer."""
     uni = not hasattr(rnn, "weight_ih_l0_reverse")
     if uni:
         # unidirectional layer (rnn_param["bidirectional"] = False): the kernels always run both directions of a layer
@@ -436,14 +499,22 @@ def _packed_weights(model, li, rnn, H, I, Ipad, x3, dev):
     if ent is not None and ent[0] == key:
         return ent[1]
     parts = []
+    pad = Hp is not None and Hp != H
+    Hd = Hp if pad else H
     for part in ((0, 1) if x3 else (0,)):
-        wih_p = torch.empty((8 * H, Ipad), dtype=torch.bfloat16, device=dev)
-        wihT_p = torch.empty((I, 8 * H), dtype=torch.bfloat16, device=dev)
-        whh_p = torch.empty((8 * H, H), dtype=torch.bfloat16, device=dev)
-        whhT_p = torch.empty((8 * H, H), dtype=torch.bfloat16, device=dev)
-        _call("ctcb200_pack_lstm_weights", _lib.ptr(rnn.weight_ih_l0), _lib.ptr(rnn.weight_hh_l0),
-              _lib.ptr(wih_r), _lib.ptr(whh_r), _lib.ptr(wih_p),
-              _lib.ptr(wihT_p), _lib.ptr(whh_p), _lib.ptr(whhT_p), H, I, Ipad, part, _cell_of(rnn)[1], _lib.stream())
+        wih_p = torch.empty((8 * Hd, Ipad), dtype=torch.bfloat16, device=dev)
+        wihT_p = torch.empty((I, 8 * Hd), dtype=torch.bfloat16, device=dev)
+        whh_p = torch.empty((8 * Hd, Hd), dtype=torch.bfloat16, device=dev)
+        whhT_p = torch.empty((8 * Hd, Hd), dtype=torch.bfloat16, device=dev)
+        if pad:
+            blk = i_blk if i_blk is not None else Ir
+            _call("ctcb200_pack_lstm_weights_padded", _lib.ptr(rnn.weight_ih_l0), _lib.ptr(rnn.weight_hh_l0),
+                  _lib.ptr(wih_r), _lib.ptr(whh_r), _lib.ptr(wih_p), _lib.ptr(wihT_p), _lib.ptr(whh_p), _lib.ptr(whhT_p),
+                  H, Hp, Ir, blk, Hp if i_blk is not None else blk, Ipad, part, _cell_of(rnn)[1], _lib.stream())
+        else:
+            _call("ctcb200_pack_lstm_weights", _lib.ptr(rnn.weight_ih_l0), _lib.ptr(rnn.weight_hh_l0),
+                  _lib.ptr(wih_r), _lib.ptr(whh_r), _lib.ptr(wih_p),
+                  _lib.ptr(wihT_p), _lib.ptr(whh_p), _lib.ptr(whhT_p), H, I, Ipad, part, _cell_of(rnn)[1], _lib.stream())
         parts.append((wih_p, wihT_p, whh_p, whhT_p))
     packed = tuple(_Opnd(parts[0][i], parts[1][i] if x3 else None) for i in range(4))
     cache[li] = (key, packed)
@@ -467,11 +538,14 @@ class _RnnStackFn(torch.autograd.Function):
         training = model.training
         x3 = model.precision == "x3"
         R = T * N
-        H = model.rnn_param["rnn_hidden_size"]
+        H = model.rnn_param["rnn_hidden_size"]   # torch shapes
+        Hp = check_hidden(H, x3)                  # device layouts (Hp > H: zero-padded units, see device_hidden)
+        pad = Hp != H
         C = model.num_class
         D = 2 if model.rnn_param["bidirectional"] else 1   # D = 1: forward half only (see _packed_weights)
         if packed and D == 1:
             raise RuntimeError("the packed-sequence path implements bidirectional layers only")
+        cols = unit_cols(H, Hp, D, dev) if pad else None   # device column of each torch feature of a layer output
         layers = list(model.rnns.children())
         ws = _Workspace()
         ws.geom, ws.layers_n, ws.x3, ws.D = geom, len(layers), x3, D
@@ -479,7 +553,7 @@ class _RnnStackFn(torch.autograd.Function):
         ws.L = []
         stream = _lib.stream
 
-        scratch = torch.empty(_lib.lib().dll.ctcb200_lstm_scratch_bytes(N, H), dtype=torch.uint8, device=dev)
+        scratch = torch.empty(_lib.lib().dll.ctcb200_lstm_scratch_bytes(N, Hp), dtype=torch.uint8, device=dev)
         # Weight gradients contract over the T*N rows: the tensor-core GEMM takes both operands in that (MN-major) form
         # (ops.gemm_atb), so the bf16 operands the forward pass makes anyway are kept and no transposed copies are built.
         defer_t = need_grad and _overlap_enabled(model) and not packed   # overlapped weight-gradient pipeline in backward()
@@ -500,15 +574,15 @@ class _RnnStackFn(torch.autograd.Function):
         I = I0
         for li, layer in enumerate(layers):
             rec = _Workspace()
-            rec.I = I
+            rec.I = rec.Ir = I
             rec.bn = None
             layer_bn = _unwrap(layer.batch_norm)
             if li > 0:
-                I = D * H
-                rec.I = I
+                I = D * Hp
+                rec.I, rec.Ir = I, D * H
                 h_prev_r = _realign(h_prev, lengths, T, N, I, 0, -1) if packed else None
                 if layer_bn is not None:
-                    rec.bn = _bn_prepare(layer_bn, h_prev, R, I, training, n_valid)
+                    rec.bn = _bn_prepare(layer_bn, h_prev, R, I, training, n_valid, cols)
                     sc_, sh_ = rec.bn.scale, rec.bn.shift
                 else:
                     sc_ = sh_ = None
@@ -517,39 +591,40 @@ class _RnnStackFn(torch.autograd.Function):
                     Xr, _ = _cast_t(h_prev_r, N * I, I, N, R, I, sc_, sh_, True, False, x3)
                     del h_prev_r
             Ipad = _round_up(I, 8)
-            wih_p, wihT_p, whh_p, whhT_p = _packed_weights(model, li, layer.rnn, H, I, Ipad, x3, dev)
+            wih_p, wihT_p, whh_p, whhT_p = _packed_weights(model, li, layer.rnn, H, I, Ipad, x3, dev, Hp, rec.Ir,
+                                                           H if li > 0 else None)
             cell, G = _cell_of(layer.rnn)
             rec.cell, rec.G = cell, G
-            hout = torch.empty((R, 2 * H), dtype=torch.float32, device=dev)
-            c_save = torch.empty((R, 2 * H), dtype=torch.float32, device=dev) if need_grad else None
-            gates = torch.empty((R, 2 * H, 4), dtype=torch.float32 if x3 else torch.float16, device=dev) if need_grad else None
-            plan = _gx_stream_plan(model, T, N, H, x3, cell, packed, dev)
+            hout = torch.empty((R, 2 * Hp), dtype=torch.float32, device=dev)
+            c_save = torch.empty((R, 2 * Hp), dtype=torch.float32, device=dev) if need_grad else None
+            gates = torch.empty((R, 2 * Hp, 4), dtype=torch.float32 if x3 else torch.float16, device=dev) if need_grad else None
+            plan = _gx_stream_plan(model, T, N, Hp, x3, cell, packed, dev)
             if plan is None:
                 if packed:   # each direction's input projection on its own alignment, written into its half of gx
-                    gx = torch.empty((R, 8 * H), dtype=torch.float32, device=dev)
-                    _gemm(X, wih_p.rows(0, 4 * H), out=gx[:, :4 * H], k=I)
-                    _gemm(Xr, wih_p.rows(4 * H, 8 * H), out=gx[:, 4 * H:], k=I)
+                    gx = torch.empty((R, 8 * Hp), dtype=torch.float32, device=dev)
+                    _gemm(X, wih_p.rows(0, 4 * Hp), out=gx[:, :4 * Hp], k=I)
+                    _gemm(Xr, wih_p.rows(4 * Hp, 8 * Hp), out=gx[:, 4 * Hp:], k=I)
                 else:
                     gx = _gemm(X, wih_p, k=I)  # [R, 8H] f32
                 _call("ctcb200_lstm_fwd", _lib.ptr(gx), _lib.ptr(whh_p.hi), _lib.ptr(whh_p.lo), _lib.ptr(hout), _lib.ptr(c_save),
-                      _lib.ptr(gates), _lib.ptr(scratch), T, N, H, model.batch_tile, cell, stream())
+                      _lib.ptr(gates), _lib.ptr(scratch), T, N, Hp, model.batch_tile, cell, stream())
             else:
                 # streamed input projection: chunk c = the rows each direction visits in its scan steps [c*chunk_T, ...)
                 chunks, chunk_T, side_ctas, mode = plan
-                gx = torch.empty((R, 8 * H), dtype=torch.float32, device=dev)
+                gx = torch.empty((R, 8 * Hp), dtype=torch.float32, device=dev)
 
                 def _gx_chunk(c, mc):
                     a, b = c * chunk_T, min(T, (c + 1) * chunk_T)
                     for d, (r0, r1) in enumerate(((a * N, b * N), ((T - b) * N, (T - a) * N))):
-                        _gemm(X.rows(r0, r1), wih_p.rows(d * 4 * H, (d + 1) * 4 * H), out=gx[r0:r1, d * 4 * H:(d + 1) * 4 * H],
-                              k=I, max_ctas=mc)
+                        _gemm(X.rows(r0, r1), wih_p.rows(d * 4 * Hp, (d + 1) * 4 * Hp),
+                              out=gx[r0:r1, d * 4 * Hp:(d + 1) * 4 * Hp], k=I, max_ctas=mc)
 
                 _gx_chunk(0, 0)
                 if mode == "serial":
                     for c in range(1, chunks):
                         _gx_chunk(c, 0)
                     _call("ctcb200_lstm_fwd", _lib.ptr(gx), _lib.ptr(whh_p.hi), _lib.ptr(whh_p.lo), _lib.ptr(hout),
-                          _lib.ptr(c_save), _lib.ptr(gates), _lib.ptr(scratch), T, N, H, model.batch_tile, cell, stream())
+                          _lib.ptr(c_save), _lib.ptr(gates), _lib.ptr(scratch), T, N, Hp, model.batch_tile, cell, stream())
                 else:
                     main_s, side_s = torch.cuda.current_stream(dev), _side_stream(dev)
                     res, rdy = _resident_state(dev), _gx_ready_state(dev)
@@ -558,7 +633,7 @@ class _RnnStackFn(torch.autograd.Function):
                     x_ready = torch.cuda.Event()
                     x_ready.record(main_s)
                     _call("ctcb200_lstm_fwd_streamed", _lib.ptr(gx), _lib.ptr(whh_p.hi), _lib.ptr(whh_p.lo), _lib.ptr(hout),
-                          _lib.ptr(c_save), _lib.ptr(gates), _lib.ptr(scratch), T, N, H, model.batch_tile, cell,
+                          _lib.ptr(c_save), _lib.ptr(gates), _lib.ptr(scratch), T, N, Hp, model.batch_tile, cell,
                           _lib.ptr(res[0]), _lib.ptr(rdy[0]), base, chunk_T, stream())
                     res[1] = (res[1] + 1) & 0xFFFFFFFF
                     with torch.cuda.stream(side_s):
@@ -575,17 +650,19 @@ class _RnnStackFn(torch.autograd.Function):
             # dW_hh pairs dG_t with the *pre-dropout* h_{t-1}: its bf16 copy can only be left to the backward pass when hout
             # is not modified in place
             if need_grad and training and p_drop > 0.0 and not packed:
-                rec.Hb, _ = _cast_t(hout, N * 2 * H, 2 * H, N, R, 2 * H, want=True, want_t=False, x3=x3)
+                rec.Hb, _ = _cast_t(hout, N * 2 * Hp, 2 * Hp, N, R, 2 * Hp, want=True, want_t=False, x3=x3)
             rec.h_out = hout if need_grad else None
             if packed:
                 # kernel alignment (forward half left-, reverse half right-aligned, garbage in the padding) -> left-aligned
                 # layer output with zero padding: what pad_packed_sequence would show (my_863_corpus/steps/model.py:93-141)
-                hout = _realign(hout, lengths, T, N, 2 * H, H, 1)
+                hout = _realign(hout, lengths, T, N, 2 * Hp, Hp, 1)
             if D == 1:
-                hout = hout[:, :H].contiguous()    # the layer's output is the forward half
+                hout = hout[:, :Hp].contiguous()    # the layer's output is the forward half
             rec.mask = None
             if training and p_drop > 0.0:
-                rec.mask = _dropout_mask(model, hout.shape, p_drop, dev)
+                rec.mask = _dropout_mask(model, (R, D * H), p_drop, dev)   # drawn in torch's shape whatever the layout
+                if pad:
+                    rec.mask = pad_cols(rec.mask, cols, D * Hp).to(torch.uint8)
                 _call("ctcb200_dropout_apply", _lib.ptr(hout), _lib.ptr(rec.mask), _inv_keep(p_drop), hout.numel(), stream())
             rec.h_in = h_prev
             rec.Xb = X if need_grad else None
@@ -595,15 +672,16 @@ class _RnnStackFn(torch.autograd.Function):
             h_prev = hout
 
         # output layer: (BatchNorm1d) + Linear(no bias) + LogSoftmax
-        F2 = D * H
+        F2 = D * Hp
         fc = _unwrap(model.fc)
         fc_bn, fc_lin = (fc[0], fc[1]) if isinstance(fc, nn.Sequential) else (None, fc)
         C = fc_lin.weight.shape[0]
-        ws.fc_bn = _bn_prepare(fc_bn, h_prev, R, F2, training, n_valid) if fc_bn is not None else None
+        ws.fc_bn = _bn_prepare(fc_bn, h_prev, R, F2, training, n_valid, cols) if fc_bn is not None else None
         Xfc, _ = _cast_t(h_prev, N * F2, F2, N, R, F2, ws.fc_bn.scale if ws.fc_bn else None,
                             ws.fc_bn.shift if ws.fc_bn else None, True, False, x3)
         ws.Xfc = Xfc if need_grad else None
-        Wfc_b, WfcT_b = _cast_t(fc_lin.weight, F2, F2, 1, C, F2, want=True, want_t=need_grad, x3=x3)
+        Wfc = pad_cols(fc_lin.weight, cols, F2) if pad else fc_lin.weight   # zero columns for the padding units
+        Wfc_b, WfcT_b = _cast_t(Wfc, F2, F2, 1, C, F2, want=True, want_t=need_grad, x3=x3)
         logits = _gemm(Xfc, Wfc_b, k=F2)  # [R, C]
         if packed:   # after pad_packed_sequence every padded frame is a zero vector
             if logits.stride(0) != C:
@@ -615,7 +693,7 @@ class _RnnStackFn(torch.autograd.Function):
             out = torch.empty((T, N, C), dtype=torch.float32, device=dev)
             _call("ctcb200_log_softmax_fwd", _lib.ptr(logits), logits.stride(0), _lib.ptr(out), R, C, stream())
         ws.h_last, ws.WfcT_b, ws.out = h_prev, WfcT_b, out
-        ws.T, ws.N, ws.H, ws.C, ws.R = T, N, H, C, R
+        ws.T, ws.N, ws.H, ws.Hp, ws.C, ws.R, ws.cols = T, N, H, Hp, C, R, cols
         ctx.ws = ws if need_grad else None
         ctx.model = model
         ctx.param_list = params
@@ -626,13 +704,14 @@ class _RnnStackFn(torch.autograd.Function):
         ws, model = ctx.ws, ctx.model
         if ws is None:
             raise RuntimeError("backward through a forward pass that ran without gradient bookkeeping")
-        T, N, H, C, R = ws.T, ws.N, ws.H, ws.C, ws.R
+        T, N, H, C, R = ws.T, ws.N, ws.H, ws.C, ws.R   # H: torch shapes
+        Hp, cols = ws.Hp, ws.cols                      # Hp: device layouts (cols: see unit_cols; None when Hp = H)
         x3, D = ws.x3, ws.D
         lengths, n_valid = ws.lengths, ws.n_valid
         packed = lengths is not None
         dev = g_out.device
         stream = _lib.stream
-        F2 = D * H
+        F2, F2r = D * Hp, D * H
         layers = list(model.rnns.children())
         grads = {}
         grad_x = None
@@ -646,7 +725,7 @@ class _RnnStackFn(torch.autograd.Function):
             res = _resident_state(dev)
             gate_ev, gate_ev_ptr = _resident_event(dev)
             side_ctas = max(8, torch.cuda.get_device_properties(dev).multi_processor_count
-                            - int(_lib.lib().dll.ctcb200_lstm_bwd_ctas(N, H, model.batch_tile)))
+                            - int(_lib.lib().dll.ctcb200_lstm_bwd_ctas(N, Hp, model.batch_tile)))
             if os.environ.get("CTCB200_SIDE_CTAS"):   # measurements: fewer CTAs for the side-stream GEMMs
                 side_ctas = max(8, min(side_ctas, int(os.environ["CTCB200_SIDE_CTAS"])))
 
@@ -670,8 +749,12 @@ class _RnnStackFn(torch.autograd.Function):
         dLb, _ = _cast_t(dlogits, N * C, C, N, R, C, want=True, want_t=False, x3=x3)
         fc = _unwrap(model.fc)
         fc_bn, fc_lin = (fc[0], fc[1]) if isinstance(fc, nn.Sequential) else (None, fc)
-        fc_buf, fc_views = _flat([C * F2] + ([F2, F2] if fc_bn is not None else []))
-        grads[fc_lin.weight] = _gemm_atb(dLb.cols(0, C), ws.Xfc.cols(0, F2), out=fc_views[0].view(C, F2), k=R)   # [C, 2H]
+        fc_buf, fc_views = _flat([C * F2r] + ([F2r, F2r] if fc_bn is not None else []))
+        if cols is None:
+            grads[fc_lin.weight] = _gemm_atb(dLb.cols(0, C), ws.Xfc.cols(0, F2), out=fc_views[0].view(C, F2), k=R)   # [C, 2H]
+        else:   # padded layout: the torch columns of the product
+            grads[fc_lin.weight] = torch.index_select(_gemm_atb(dLb.cols(0, C), ws.Xfc.cols(0, F2), k=R), 1, cols,
+                                                      out=fc_views[0].view(C, F2r))
         dh = _gemm(dLb, ws.WfcT_b, k=C)                                                # [R, 2H]
         dws = torch.empty(2 * F2, dtype=torch.float64, device=dev)
         fuse_env = os.environ.get("CTCB200_BN_FUSE", "1") != "0"
@@ -679,12 +762,23 @@ class _RnnStackFn(torch.autograd.Function):
         def _bn_backward(bn_mod, st, dy, x_in, C_, below, dgam, dbet):
             """BatchNorm1d backward of `bn_mod` for gradient dy [R, C_] w.r.t. its output; x_in is its input (the output of the
             layer below). Returns (bn_x, bn_coef) when the input gradient is left to the BPTT kernel of that layer (no dropout
-            mask in between), else applies it in place and returns None."""
+            mask in between), else applies it in place and returns None. Padded layout: the kernels see the padded parameter
+            image of _bn_prepare, dgam / dbet receive the torch columns."""
             grads[bn_mod.weight], grads[bn_mod.bias] = dgam, dbet
+            if st.cols is None:
+                return _bn_backward_dev(st, dy, x_in, C_, below, dgam, dbet)
+            dgam_p = torch.empty(C_, dtype=torch.float32, device=dev)
+            dbet_p = torch.empty(C_, dtype=torch.float32, device=dev)
+            fused = _bn_backward_dev(st, dy, x_in, C_, below, dgam_p, dbet_p)
+            torch.index_select(dgam_p, 0, st.cols, out=dgam)
+            torch.index_select(dbet_p, 0, st.cols, out=dbet)
+            return fused
+
+        def _bn_backward_dev(st, dy, x_in, C_, below, dgam, dbet):
             if ((fuse_env and ws.L[below].mask is None and D == 2) or not st.batch) and not (packed and st.batch):
                 coef = torch.empty(3 * C_, dtype=torch.float32, device=dev)
                 _call("ctcb200_bn_bwd_coef", _lib.ptr(dy), _lib.ptr(x_in), _lib.ptr(st.mean), _lib.ptr(st.rstd),
-                      _lib.ptr(bn_mod.weight), _lib.ptr(coef), _lib.ptr(dgam), _lib.ptr(dbet), R, C_, _lib.ptr(dws), n_valid,
+                      _lib.ptr(st.gamma), _lib.ptr(coef), _lib.ptr(dgam), _lib.ptr(dbet), R, C_, _lib.ptr(dws), n_valid,
                       stream())
                 if not st.batch:
                     coef[C_:].zero_()   # frozen statistics: dx = gamma * rstd * dy, no batch-coupling terms
@@ -696,7 +790,7 @@ class _RnnStackFn(torch.autograd.Function):
                 return (x_in, coef)
             # packed mode: the padding rows of dx come out non-zero here; the realign in front of the BPTT kernel zeroes them
             _call("ctcb200_bn_bwd", _lib.ptr(dy), _lib.ptr(x_in), _lib.ptr(st.mean), _lib.ptr(st.rstd),
-                  _lib.ptr(bn_mod.weight), _lib.ptr(dy), _lib.ptr(dgam), _lib.ptr(dbet), R, C_, _lib.ptr(dws), n_valid, stream())
+                  _lib.ptr(st.gamma), _lib.ptr(dy), _lib.ptr(dgam), _lib.ptr(dbet), R, C_, _lib.ptr(dws), n_valid, stream())
             return None
 
         bn_fuse = None
@@ -707,23 +801,32 @@ class _RnnStackFn(torch.autograd.Function):
 
         def _wgrad_finish(item, tmp_ih, t1, t2, extra=()):
             """Weight-gradient products (rows in dG's packed gate order) -> torch's layout inside the layer's flat bucket; hands
-            the bucket to the gradient all-reduce."""
+            the bucket to the gradient all-reduce. Padded layout: the rows of the real units (the gate-row gather works at any
+            Hp), then the torch columns (the padded input layout above the first layer, the real units of W_hh)."""
             layer_, rec_, (dg_, dgrec_), li_, buf_, views_ = item
             rnn = layer_.rnn
             GH = rec_.G * H     # rows of torch's weight matrices per direction (4H LSTM, 3H GRU, H RNN)
-            I_ = rec_.I
+            I_ = rec_.Ir
             perm = _gate_row_perm(H, dev)
+            in_cols = cols if (cols is not None and li_ > 0) else None
+            hh_cols = unit_cols(H, Hp, 1, dev) if cols is not None else None
+
+            def gather(src, out, col_idx):
+                if col_idx is None:
+                    torch.index_select(src, 0, perm, out=out)
+                else:
+                    torch.index_select(torch.index_select(src, 0, perm), 1, col_idx, out=out)
             dwih = views_[0].view(8 * H, I_)
-            torch.index_select(tmp_ih[0], 0, perm, out=dwih[:4 * H])
-            torch.index_select(tmp_ih[1], 0, perm, out=dwih[4 * H:])
+            gather(tmp_ih[0], dwih[:4 * H], in_cols)
+            gather(tmp_ih[1], dwih[4 * H:], in_cols)
             grads[rnn.weight_ih_l0] = dwih[:GH]
             whf, whr = views_[1].view(4 * H, H), views_[2].view(4 * H, H)
             if t1 is not None:
-                torch.index_select(t1, 0, perm, out=whf)
+                gather(t1, whf, hh_cols)
             else:
                 whf.zero_()
             if t2 is not None:
-                torch.index_select(t2, 0, perm, out=whr)
+                gather(t2, whr, hh_cols)
             else:
                 whr.zero_()
             grads[rnn.weight_hh_l0] = whf[:GH]
@@ -743,20 +846,20 @@ class _RnnStackFn(torch.autograd.Function):
             # BPTT kernel, layer input [R, I] bf16 from the forward pass, layer output [R, 2H] cast here
             Xb, Hb = rec_.Xb, rec_.Hb
             if Hb is None:
-                Hb, _ = _cast_t(rec_.h_out, N * 2 * H, 2 * H, N, R, 2 * H, want=True, want_t=False, x3=x3)
+                Hb, _ = _cast_t(rec_.h_out, N * 2 * Hp, 2 * Hp, N, R, 2 * Hp, want=True, want_t=False, x3=x3)
             if packed:   # each direction against the input in its own alignment
-                tmp_ih = (_gemm_atb(dg_.cols(0, 4 * H), Xb.cols(0, I_), k=R, max_ctas=mc),
-                          _gemm_atb(dg_.cols(4 * H, 8 * H), rec_.Xrb.cols(0, I_), k=R, max_ctas=mc))
+                tmp_ih = (_gemm_atb(dg_.cols(0, 4 * Hp), Xb.cols(0, I_), k=R, max_ctas=mc),
+                          _gemm_atb(dg_.cols(4 * Hp, 8 * Hp), rec_.Xrb.cols(0, I_), k=R, max_ctas=mc))
             else:
                 tmp = _gemm_atb(dg_, Xb.cols(0, I_), k=R, max_ctas=mc)                   # [8H, I]
-                tmp_ih = (tmp[:4 * H], tmp[4 * H:])
+                tmp_ih = (tmp[:4 * Hp], tmp[4 * Hp:])
             dgr_ = dgrec_ if dgrec_ is not None else dg_     # what the recurrent weights see (GRU differs)
             t1 = t2 = None
             if T > 1:
                 # pairs (dG_t, h_{t-1}) for the forward scan, (dG_t, h_{t+1}) for the reverse scan: one time step = N rows
-                t1 = _gemm_atb(dgr_.cols(0, 4 * H), Hb.cols(0, H), a_roff=N, b_roff=0, k=R - N, max_ctas=mc)
+                t1 = _gemm_atb(dgr_.cols(0, 4 * Hp), Hb.cols(0, Hp), a_roff=N, b_roff=0, k=R - N, max_ctas=mc)
                 if D == 2:
-                    t2 = _gemm_atb(dgr_.cols(4 * H, 8 * H), Hb.cols(H, 2 * H), a_roff=0, b_roff=N, k=R - N, max_ctas=mc)
+                    t2 = _gemm_atb(dgr_.cols(4 * Hp, 8 * Hp), Hb.cols(Hp, 2 * Hp), a_roff=0, b_roff=N, k=R - N, max_ctas=mc)
             _wgrad_finish(item, tmp_ih, t1, t2, (Xb, Hb))
 
         # ---- streamed gate gradients (_dg_stream_plan): chunk c = scan steps [c*chunk_T, (c+1)*chunk_T) of both BPTT scans ----
@@ -767,52 +870,53 @@ class _RnnStackFn(torch.autograd.Function):
         def _dx_chunk(dg_, rec_, dx_, c, chunk_T, mc):
             """this chunk's share of dX = dG W_ih: each direction's K half against the rows it has finished (accumulated)."""
             for d, (ta, tb) in enumerate(_chunk_frames(c, chunk_T)):
-                _gemm(dg_.rows(ta * N, tb * N), rec_.wihT_p, out=dx_[ta * N:tb * N], k=4 * H, a_koff=d * 4 * H, b_koff=d * 4 * H,
-                      accumulate=True, max_ctas=mc)
+                _gemm(dg_.rows(ta * N, tb * N), rec_.wihT_p, out=dx_[ta * N:tb * N], k=4 * Hp, a_koff=d * 4 * Hp,
+                      b_koff=d * 4 * Hp, accumulate=True, max_ctas=mc)
 
         def _wg_chunk(st, c, chunk_T, mc):
             """this chunk's share of the first layer's dW_ih / dW_hh contractions over time (accumulated)."""
             dg_, dgr_, Xb, Hb, I_, tmp_ih, t1, t2 = st
             (fa, fb), (ra, rb) = _chunk_frames(c, chunk_T)
-            _gemm_atb(dg_.cols(0, 4 * H), Xb.cols(0, I_), out=tmp_ih[0], accumulate=True, a_roff=fa * N, b_roff=fa * N,
+            _gemm_atb(dg_.cols(0, 4 * Hp), Xb.cols(0, I_), out=tmp_ih[0], accumulate=True, a_roff=fa * N, b_roff=fa * N,
                       k=(fb - fa) * N, max_ctas=mc)
-            _gemm_atb(dg_.cols(4 * H, 8 * H), Xb.cols(0, I_), out=tmp_ih[1], accumulate=True, a_roff=ra * N, b_roff=ra * N,
+            _gemm_atb(dg_.cols(4 * Hp, 8 * Hp), Xb.cols(0, I_), out=tmp_ih[1], accumulate=True, a_roff=ra * N, b_roff=ra * N,
                       k=(rb - ra) * N, max_ctas=mc)
             f0 = max(fa, 1)           # (dG_t, h_{t-1}), t >= 1
             if fb > f0:
-                _gemm_atb(dgr_.cols(0, 4 * H), Hb.cols(0, H), out=t1, accumulate=True, a_roff=f0 * N, b_roff=(f0 - 1) * N,
+                _gemm_atb(dgr_.cols(0, 4 * Hp), Hb.cols(0, Hp), out=t1, accumulate=True, a_roff=f0 * N, b_roff=(f0 - 1) * N,
                           k=(fb - f0) * N, max_ctas=mc)
             r1 = min(rb, T - 1)       # (dG_t, h_{t+1}), t <= T - 2
             if r1 > ra:
-                _gemm_atb(dgr_.cols(4 * H, 8 * H), Hb.cols(H, 2 * H), out=t2, accumulate=True, a_roff=ra * N, b_roff=(ra + 1) * N,
-                          k=(r1 - ra) * N, max_ctas=mc)
+                _gemm_atb(dgr_.cols(4 * Hp, 8 * Hp), Hb.cols(Hp, 2 * Hp), out=t2, accumulate=True, a_roff=ra * N,
+                          b_roff=(ra + 1) * N, k=(r1 - ra) * N, max_ctas=mc)
 
         pending = None
-        scratch = torch.empty(_lib.lib().dll.ctcb200_lstm_scratch_bytes(N, H), dtype=torch.uint8, device=dev)
+        scratch = torch.empty(_lib.lib().dll.ctcb200_lstm_scratch_bytes(N, Hp), dtype=torch.uint8, device=dev)
         for li in range(len(layers) - 1, -1, -1):
             layer, rec = layers[li], ws.L[li]
             I = rec.I
             layer_bn = _unwrap(layer.batch_norm)
             has_bn = li > 0 and layer_bn is not None
-            buf, views = _flat([8 * H * I, 4 * H * H, 4 * H * H] + ([I, I] if has_bn else []))
+            Ir = rec.Ir
+            buf, views = _flat([8 * H * Ir, 4 * H * H, 4 * H * H] + ([Ir, Ir] if has_bn else []))   # torch shapes
             if rec.mask is not None:
                 _call("ctcb200_dropout_apply", _lib.ptr(dh), _lib.ptr(rec.mask), _inv_keep(_layer_dropout_p(layer)),
                       dh.numel(), stream())
             if packed:   # left-aligned gradient -> the kernels' alignment (reverse half right-aligned), padding rows zeroed
-                dh = _realign(dh, lengths, T, N, 2 * H, H, -1)
+                dh = _realign(dh, lengths, T, N, 2 * Hp, Hp, -1)
             if D == 1:   # forward half only: the kernel still takes a [R, 2H] gradient, the reverse half gets none
-                dh2 = torch.zeros((R, 2 * H), dtype=torch.float32, device=dev)
-                dh2[:, :H].copy_(dh)
+                dh2 = torch.zeros((R, 2 * Hp), dtype=torch.float32, device=dev)
+                dh2[:, :Hp].copy_(dh)
                 dh = dh2
             def _dg_buf():
                 # unused gate slots of GRU / RNN layers are never written by the kernel: they must read as zero
                 alloc = torch.empty if rec.G == 4 else torch.zeros
-                return _Opnd(alloc((R, 8 * H), dtype=torch.bfloat16, device=dev),
-                             alloc((R, 8 * H), dtype=torch.bfloat16, device=dev) if x3 else None)
+                return _Opnd(alloc((R, 8 * Hp), dtype=torch.bfloat16, device=dev),
+                             alloc((R, 8 * Hp), dtype=torch.bfloat16, device=dev) if x3 else None)
             dg = _dg_buf()
             dg_rec = _dg_buf() if rec.cell == 1 else None   # GRU: the recurrent weights see a different n-gate gradient
             need_dx = li > 0 or bool(ctx.needs_input_grad[1])
-            plan = _dg_stream_plan(model, T, N, H, D, x3, rec.cell, packed, overlap and gate == "memop", dev)
+            plan = _dg_stream_plan(model, T, N, Hp, D, x3, rec.cell, packed, overlap and gate == "memop", dev)
             streamed = plan is not None and plan[3] == "stream"
             dx_s = wg0 = None
             if plan is not None:
@@ -822,13 +926,13 @@ class _RnnStackFn(torch.autograd.Function):
                 if need_dx:
                     dx_s = torch.zeros((R, I), dtype=torch.float32, device=dev)
                 if li == 0:   # the first layer's weight gradients have no later BPTT kernel to hide under
-                    tmp0 = torch.zeros((8 * H, I), dtype=torch.float32, device=dev)
-                    wg0 = [dg, dg_rec if dg_rec is not None else dg, rec.Xb, rec.Hb, I, (tmp0[:4 * H], tmp0[4 * H:]),
-                           torch.zeros((4 * H, H), dtype=torch.float32, device=dev),
-                           torch.zeros((4 * H, H), dtype=torch.float32, device=dev)]
+                    tmp0 = torch.zeros((8 * Hp, I), dtype=torch.float32, device=dev)
+                    wg0 = [dg, dg_rec if dg_rec is not None else dg, rec.Xb, rec.Hb, I, (tmp0[:4 * Hp], tmp0[4 * Hp:]),
+                           torch.zeros((4 * Hp, Hp), dtype=torch.float32, device=dev),
+                           torch.zeros((4 * Hp, Hp), dtype=torch.float32, device=dev)]
             bwd_args = (_lib.ptr(dh), _lib.ptr(rec.whhT_p.hi), _lib.ptr(rec.whhT_p.lo), _lib.ptr(rec.c_save),
                         _lib.ptr(rec.gates), _lib.ptr(dg.hi), _lib.ptr(dg.lo), _lib.ptr(dg_rec.hi) if dg_rec else None,
-                        _lib.ptr(dg_rec.lo) if dg_rec else None, _lib.ptr(scratch), T, N, H, model.batch_tile, rec.cell,
+                        _lib.ptr(dg_rec.lo) if dg_rec else None, _lib.ptr(scratch), T, N, Hp, model.batch_tile, rec.cell,
                         _lib.ptr(bn_fuse[0]) if bn_fuse else None, _lib.ptr(bn_fuse[1]) if bn_fuse else None,
                         _lib.ptr(res[0]) if (overlap and gate == "memop") else None)
             if streamed:
@@ -873,7 +977,7 @@ class _RnnStackFn(torch.autograd.Function):
             if plan is not None:
                 if wg0 is not None and wg0[3] is None:
                     with torch.cuda.stream(side) if streamed else contextlib.nullcontext():
-                        wg0[3], _ = _cast_t(rec.h_out, N * 2 * H, 2 * H, N, R, 2 * H, want=True, want_t=False, x3=x3)
+                        wg0[3], _ = _cast_t(rec.h_out, N * 2 * Hp, 2 * Hp, N, R, 2 * Hp, want=True, want_t=False, x3=x3)
                 if streamed:
                     with torch.cuda.stream(side):
                         _chunks_of(range(chunks - 1), side_ctas)
@@ -888,9 +992,9 @@ class _RnnStackFn(torch.autograd.Function):
                 if dx_s is not None:
                     return dx_s
                 if not packed:
-                    return _gemm(dg, rec.wihT_p, k=8 * H)                  # [R, I] rows (t, n)
-                dxf = _gemm(dg, rec.wihT_p, k=4 * H)                       # forward direction: already left-aligned
-                dxr = _gemm(dg, rec.wihT_p, k=4 * H, a_koff=4 * H, b_koff=4 * H)
+                    return _gemm(dg, rec.wihT_p, k=8 * Hp)                  # [R, I] rows (t, n)
+                dxf = _gemm(dg, rec.wihT_p, k=4 * Hp)                       # forward direction: already left-aligned
+                dxr = _gemm(dg, rec.wihT_p, k=4 * Hp, a_koff=4 * Hp, b_koff=4 * Hp)
                 return _realign(dxr, lengths, T, N, I, 0, 1, dst=dxf, accumulate=True)
             if li == 0 and ctx.needs_input_grad[1]:
                 dx0 = _input_grad()
@@ -991,6 +1095,7 @@ class CTC_Model(nn.Module):
             raise RuntimeError("model parameters and input must live on the same CUDA device")
         if self.precision not in ("bf16", "x3"):
             raise RuntimeError("CTC_Model.precision must be 'bf16' or 'x3' (got %r)" % (self.precision,))
+        check_hidden(self.rnn_param["rnn_hidden_size"], self.precision == "x3")
 
     def _rnn_params(self):
         plist = []

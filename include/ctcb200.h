@@ -130,7 +130,11 @@ CTCB200_API int ctcb200_gemm_atb_bf16(const void* A, int64_t lda, const void* B,
  * non-NULL the layer output feeds a training-mode BatchNorm1d (model_ctc.py:29-32) whose backward is applied on the fly:
  * dhout is then the gradient w.r.t. the normalised tensor, bn_x f32 [T*N, 2H] the layer output itself and
  * bn_coef f32 [3][2H] comes from ctcb200_bn_bwd_coef.
- * batch_tile: 0 = auto, or 16 / 32 batch columns per CTA group. H must be a multiple of 128, <= 640. */
+ * batch_tile: 0 = auto, or 16 / 32 batch columns per CTA group. The recurrent entry points take the DEVICE hidden size: a multiple
+ * of 128 in [128, 1024], at most 640 in the split-operand mode. Above 640 the kernels exchange h_t / dG_t through global memory
+ * with cooperative launches (no streamed projection / gate gradients: ctcb200_lstm_fwd_ctas / _bwd_plan return 0). Any other
+ * hidden size H runs at Hp = 128 * ceil(H / 128) with zero padding (ctcb200_pack_lstm_weights_padded): the Hp - H extra units
+ * keep h = c = 0 exactly and every activation / gradient buffer uses the Hp layout. */
 CTCB200_API int64_t ctcb200_lstm_scratch_bytes(int N, int H);
 /* Split-operand ("x3") precision mode — fp32-grade results from bf16 tensor-core products, for parity with the reference's
  * fp32 nn.LSTM arithmetic (model_ctc.py:23-26) to 1e-3 on every gradient: each fp32 operand v is carried as two bf16 tensors,
@@ -146,6 +150,16 @@ CTCB200_API int64_t ctcb200_lstm_scratch_bytes(int N, int H);
 CTCB200_API int ctcb200_pack_lstm_weights(const float* wih_f, const float* whh_f, const float* wih_r,
                                           const float* whh_r, void* wih_p, void* wihT_p, void* whh_p, void* whhT_p,
                                           int H, int I, int Ipad, int part, int gates, ctcb200_stream_t stream);
+/* Zero-padded packing for a torch hidden size H run at the device hidden size Hp >= H (Hp a multiple of 128 for the recurrent
+ * kernels): the same layouts at Hp — wih_p [8Hp, Ipad], wihT_p [I_dev, 8Hp], whh_p / whhT_p [8Hp, Hp] — with zero rows for the
+ * units >= H and zero recurrent columns for them. The torch input columns come in blocks of i_blk that sit i_blk_p apart on the
+ * device (a layer above a padded one: i_blk = H, i_blk_p = Hp; the first layer: i_blk = i_blk_p = I), so
+ * I_dev = (I / i_blk) * i_blk_p <= Ipad, and the device columns between the blocks are zero. H = Hp with i_blk = i_blk_p gives
+ * exactly ctcb200_pack_lstm_weights. */
+CTCB200_API int ctcb200_pack_lstm_weights_padded(const float* wih_f, const float* whh_f, const float* wih_r,
+                                                 const float* whh_r, void* wih_p, void* wihT_p, void* whh_p, void* whhT_p,
+                                                 int H, int Hp, int I, int i_blk, int i_blk_p, int Ipad, int part, int gates,
+                                                 ctcb200_stream_t stream);
 CTCB200_API int ctcb200_lstm_fwd(const float* gx, const void* whh_packed, const void* whh_lo_packed, float* hout,
                                  float* c_save, void* gates_save, void* scratch, int T, int N, int H, int batch_tile,
                                  int cell, ctcb200_stream_t stream);
